@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline measurement of the geometry path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config B of SURVEY.md section 8d, `configs[1]` of BASELINE.json): one synthetic 1M-face
 terrain mesh per GPU, the canonical 6-view orthographic rig, 768x768, outputs mask + position +
@@ -33,6 +33,10 @@ JSON keys beyond the base contract:
 `--impl reference` times the reference's render path on the host cores.  The reference has no CPU
 implementation of its own (its rasterizer is the GPU-only nvdiffrast), so this arm is the oracle
 port: the reference's Python restated in NumPy over the C/OpenMP restatement of the operators.
+
+`--dump-outputs DIR` writes the four maps of the last timed step (rank 0's mesh) as DIR/{mask,pos,depth,normal}.npy,
+float32, at a fixed sample of pixels (see dump_outputs); the inputs are seeded, so two builds, or the two arms, can be
+compared file by file.
 """
 from __future__ import annotations
 
@@ -54,6 +58,21 @@ N_VIEWS = 6
 TERRAIN = (1000, 500)  # quads -> 1 000 000 faces, 501 501 vertices
 METRIC = "views_per_sec_768sq_pos_normal_1M_face_mesh"
 UNIT = "views/s"
+MAPS = ("mask", "pos", "depth", "normal")   # what render() returns to the caller of the timed step
+DUMP_PIXELS = 1 << 20                       # 32 MiB of float32 for the four maps (a step has 3.5 M pixels, 113 MB)
+
+
+def dump_outputs(dump_dir: str, maps: dict) -> None:
+    """Writes each map (torch tensor or NumPy array, leading dims views x H x W) as DIR/<name>.npy in float32, the mask
+    as 0 / 1, at the same DUMP_PIXELS (view, y, x) positions: drawn with seed 0 without replacement, in increasing
+    flat order.  pos and normal keep their channel axis: (DUMP_PIXELS, 3)."""
+    os.makedirs(dump_dir, exist_ok=True)
+    n_pix = N_VIEWS * H * W
+    idx = np.sort(np.random.default_rng(0).choice(n_pix, DUMP_PIXELS, replace=False))
+    for name, m in maps.items():
+        a = m.cpu().numpy() if hasattr(m, "cpu") else np.asarray(m)
+        a = a.reshape(n_pix, -1)[idx].reshape((DUMP_PIXELS,) + a.shape[3:])
+        np.save(os.path.join(dump_dir, f"{name}.npy"), a.astype(np.float32))
 
 
 def terrain_arrays(seed: int):
@@ -179,8 +198,10 @@ def run_reference(args):
         cpu_render_step(state)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_render_step(state)
+        out = cpu_render_step(state)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {name: out[name] for name in MAPS})
     value = N_VIEWS * args.steps / dt
     cores = cpu_threads()
     line = {
@@ -280,6 +301,8 @@ def run_ours(args):
             stops[k].record()
         barrier()
         t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {name: getattr(out, name) for name in MAPS})
     step_ms = [starts[k].elapsed_time(stops[k]) for k in range(K)]
     total_ms = float(sum(step_ms))
     tot = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -855,10 +878,11 @@ def main():
     ap.add_argument("--no-extra", action="store_true", help="skip config D and the config E sharded bake")
     ap.add_argument("--small-e", action="store_true", help="config E at the scaled shape (1M faces, 32 x 1024^2, 2048^2 atlas)")
     ap.add_argument("--eager", action="store_true", help="time the eager render() call instead of its CUDA-graph replay")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the maps of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
-        if args.steps > 40:
-            args.steps = 40  # each step is ~0.1-1 s of host work; keep the arm within minutes
         run_reference(args)
     else:
         run_ours(args)

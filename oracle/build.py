@@ -10,9 +10,12 @@ so nothing of the reference can be compiled here (recorded in DESIGN.md section 
 """
 from __future__ import annotations
 
+import atexit
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SRCS = [os.path.join(HERE, "wr_oracle.c"), os.path.join(HERE, "wr_oracle_blend.c")]
@@ -45,14 +48,21 @@ LIB = os.path.join(OUT_DIR, f"libwr_oracle_{_host_tag()}.so")
 
 
 def build(force: bool = False) -> str:
-    os.makedirs(OUT_DIR, exist_ok=True)
     if not force and os.path.exists(LIB) and os.path.getmtime(LIB) >= max(os.path.getmtime(p) for p in SRCS):
         return LIB
-    tmp = LIB + f".{os.getpid()}.tmp"   # several ranks may build at once: write aside, then rename atomically
+    lib = LIB
+    if not os.access(OUT_DIR if os.path.isdir(OUT_DIR) else HERE, os.W_OK):
+        # A read-only tree (bench.py may run from one) on a host without a build for its CPU: build into a directory
+        # private to this process (mkdtemp: mode 0700, a fresh name), never reused and removed at exit.
+        out = tempfile.mkdtemp(prefix="wr_oracle_")
+        atexit.register(shutil.rmtree, out, True)
+        lib = os.path.join(out, os.path.basename(LIB))
+    os.makedirs(os.path.dirname(lib), exist_ok=True)
+    tmp = lib + f".{os.getpid()}.tmp"   # several ranks may build at once: write aside, then rename atomically
     cmd = ["gcc", *CFLAGS, *SRCS, "-o", tmp, "-lm"]
     subprocess.run(cmd, check=True)
-    os.replace(tmp, LIB)
-    return LIB
+    os.replace(tmp, lib)
+    return lib
 
 
 if __name__ == "__main__":
