@@ -133,6 +133,42 @@ def perspective_cameras(n: int = 4, fovy: float = 40.0, distance: float = 1.8, d
                          azimuth_deg=[0.0, 75.0, 160.0, 250.0][:n], device=device)
 
 
+def concat_cameras(*cams):
+    """One rig from parts (views in argument order)."""
+    import torch
+    import worldrenderer_b200 as wr
+    return wr.Camera(**{k: torch.cat([getattr(c, k) for c in cams]).contiguous()
+                        for k in ("c2w", "w2c", "proj_mtx", "mvp_mtx", "cam_pos")})
+
+
+def bake_perspective_cameras(H: int, W: int, device=None):
+    """perspective_cameras() with the image aspect of an H x W view, as CameraProjection(cam=None) builds it."""
+    import worldrenderer_b200 as wr
+    return wr.get_camera(elevation_deg=[10.0, -20.0, 35.0, 60.0], distance=[1.8] * 4, fovy_deg=[40.0] * 4,
+                         azimuth_deg=[0.0, 75.0, 160.0, 250.0], aspect_wh=W / H, device=device)
+
+
+def mixed_40_view_cameras(H: int, W: int, device=None):
+    """40 views: 34 perspective and the 6 canonical orthographic ones.  Orthographic views sit at indices 1-3 (the
+    unit-row fast path of the unprojection) and 37-39 (beyond the 32-view bitmask: the general path); the perspective
+    views 33-35 would read the bits of views 1-3 from a bitmask indexed by v & 31 instead of tested for v < 32."""
+    import worldrenderer_b200 as wr
+    n = 34
+    persp = wr.get_camera(elevation_deg=np.linspace(-60.0, 70.0, n).tolist(), distance=[1.8] * n,
+                          fovy_deg=[40.0] * n, azimuth_deg=((np.arange(n) * 137.5) % 360.0).tolist(),
+                          aspect_wh=W / H, device=device)
+    ortho = canonical_cameras(device=device)
+    return concat_cameras(persp[0:1], ortho[0:3], persp[1:34], ortho[3:6])
+
+
+def low_terrain_cameras(H: int, W: int, device=None):
+    """Two wide perspective cameras close over the terrain_mesh: much of the terrain lies behind them (clip w <= 0,
+    NDC up to ~1e5), which the bake projects without a w > 0 guard."""
+    import worldrenderer_b200 as wr
+    return wr.get_camera(elevation_deg=[60.0, 60.0], distance=[0.25, 0.25], fovy_deg=[110.0, 110.0],
+                         azimuth_deg=[0.0, 120.0], near=0.01, aspect_wh=W / H, device=device)
+
+
 def inside_cameras(device=None):
     """Perspective cameras placed INSIDE the mesh's bounding sphere: triangles cross the near plane."""
     import worldrenderer_b200 as wr

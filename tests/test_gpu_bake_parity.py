@@ -168,18 +168,25 @@ def test_fused_unprojection_with_first_view_dominate_equals_stepwise(wr_ctx):
 
 
 def test_unprojection_in_texel_ranges_equals_one_pass(wr_ctx):
-    """wr_uv_unproject over texel ranges (what the chunked multi-GPU bake issues) fills the same accumulators."""
+    """wr_uv_unproject over texel ranges (what the chunked multi-GPU bake issues) fills the same accumulators, on a
+    square and on non-square atlases: range ends inside a row, a single texel, and a range ending at a row end."""
     from worldrenderer_b200.uv import fused_unproject, fused_view_maps
     mesh, cam, images = _setup(wr_ctx.device)
-    pre = wr.uv_precompute(wr_ctx, mesh, 128, 128)
     img = torch.from_numpy(images).to(wr_ctx.device)
     kw = dict(aoi_cos_thresh=0.2, depth_grad_thresh=0.1, alpha=3.0, accumulate_only=True)
     _, geo, att = fused_view_maps(wr_ctx, mesh, cam, img, 96, 96, 5)
-    _, _, full, _, _ = fused_unproject(wr_ctx, pre, cam, 96, 96, geo, att, **kw)
-    part = torch.full_like(full, float("nan"))
-    for lo, hi in [(0, 5000), (5000, 5001), (5001, 16384)]:
-        fused_unproject(wr_ctx, pre, cam, 96, 96, geo, att, accum=part, add_to_accum=False, tex_range=(lo, hi), **kw)
-    assert torch.equal(part, full)
+    for Hu, Wu in [(128, 128), (96, 160), (160, 96)]:
+        pre = wr.uv_precompute(wr_ctx, mesh, Hu, Wu)
+        _, _, full, _, _ = fused_unproject(wr_ctx, pre, cam, 96, 96, geo, att, **kw)
+        assert full.shape == (Hu, Wu, 5) and float(full[..., 4].sum()) > 1000
+        row_end = (5001 // Wu + 1) * Wu
+        cuts = [0, 5000, 5001, row_end, row_end + 1, Hu * Wu]
+        assert 5000 % Wu and 5001 % Wu
+        part = torch.full_like(full, float("nan"))
+        for lo, hi in zip(cuts[:-1], cuts[1:]):
+            fused_unproject(wr_ctx, pre, cam, 96, 96, geo, att, accum=part, add_to_accum=False, tex_range=(lo, hi),
+                            **kw)
+        assert torch.equal(part, full), (Hu, Wu)
     with pytest.raises(RuntimeError):
         fused_unproject(wr_ctx, pre, cam, 96, 96, geo, att, accum=part, add_to_accum=False, tex_range=(10, 5), **kw)
 

@@ -147,3 +147,38 @@ def test_sizes_and_empty():
         assert (ids >= 0).all()
     r, i = shim.rasterize(np.zeros((1, 0, 4), np.float32), np.zeros((0, 3), np.int32), (4, 4))
     assert (i == -1).all() and (r == 0).all()
+
+
+@pytest.mark.parametrize("H,W,C", [(1, 17, 1), (33, 20, 3), (64, 96, 4), (7, 5, 2)])
+def test_grid_sample_matches_the_reference_operator(H, W, C):
+    """render_oracle.grid_sample (the statement wr_grid_sample and the bake kernels follow bit for bit) against
+    torch.nn.functional.grid_sample(bilinear, zeros, align_corners=False) itself, at non-square maps.
+
+    Finite coordinates: not bit-exact, because torch forms the tap weights as (x0 + 1 - ix) where the oracle has
+    1 - (ix - x0), and its pixel coordinate ix may round differently.  A shift of ix or iy by up to one ulp of the map
+    extent moves the result by at most 2 * ulp(max(H, W)) * max |tap difference| <= 4 eps max(H, W) max |img|;
+    measured up to 1.3e-5 on N(0, 1) maps of up to 64 x 96 (the bound there is 1.8e-4).
+
+    Non-finite coordinates: torch returns NaN on CPU and 0 on CUDA; the oracle (and every kernel) returns 0 -- the
+    sample adds nothing (DESIGN.md section 4)."""
+    import torch
+    import torch.nn.functional as F
+    from oracle import render_oracle
+    rng = np.random.default_rng(10 * H + W)
+    img = rng.standard_normal((H, W, C)).astype(np.float32)
+    ndc = rng.uniform(-1.3, 1.3, (23, 31, 2)).astype(np.float32)
+    def edge(n):   # the borders, one pixel in / out of them, a pixel centre, -0
+        return np.array([-1, 1, -1 - 1 / n, -1 + 1 / n, 1 - 1 / n, 1 + 1 / n, (2 * (n // 2) + 1) / n - 1, -0.0], np.float32)
+    ndc[0, :8, 0] = edge(W)
+    ndc[1, :8, 1] = edge(H)
+    got = render_oracle.grid_sample(img, ndc)
+    ref = F.grid_sample(torch.from_numpy(img).permute(2, 0, 1)[None], torch.from_numpy(ndc)[None], mode="bilinear",
+                        padding_mode="zeros", align_corners=False)[0].permute(1, 2, 0).numpy()
+    assert got.shape == (23, 31, C)
+    tol = 4 * np.finfo(np.float32).eps * max(H, W) * np.abs(img).max()
+    np.testing.assert_allclose(got, ref, rtol=0, atol=tol)
+    assert np.abs(ref).max() > 0.5   # not a field of zeros
+
+    bad = np.array([[np.nan, 0.0], [0.0, np.nan], [np.inf, 0.0], [-np.inf, 0.5], [0.25, np.inf], [0.0, -np.inf],
+                    [np.inf, np.nan]], np.float32)[None]
+    np.testing.assert_array_equal(render_oracle.grid_sample(img, bad), np.zeros((1, len(bad[0]), C), np.float32))
