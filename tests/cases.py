@@ -113,6 +113,56 @@ def icosphere_mesh(frequency: int = 8):
     return v.astype(f32), f.astype(np.int32)
 
 
+def exact_vertex_normals(v, f):
+    """Vertex normals as the GPU splats them: float face normals summed in float64 (the correctly rounded sum,
+    whatever the order), rounded to float once, normalised in float."""
+    ff = np.asarray(f, np.int64)
+    e1 = (v[ff[:, 1]] - v[ff[:, 0]]).astype(f32)
+    e2 = (v[ff[:, 2]] - v[ff[:, 0]]).astype(f32)
+    fn = np.stack([e1[:, 1] * e2[:, 2] - e1[:, 2] * e2[:, 1], e1[:, 2] * e2[:, 0] - e1[:, 0] * e2[:, 2],
+                   e1[:, 0] * e2[:, 1] - e1[:, 1] * e2[:, 0]], -1).astype(f32)
+    acc = np.zeros((v.shape[0], 3), np.float64)
+    for k in range(3):
+        np.add.at(acc, ff[:, k], fn.astype(np.float64))
+    s32 = acc.astype(f32)
+    n = s32 / np.maximum(np.sqrt((s32[:, 0] * s32[:, 0] + s32[:, 1] * s32[:, 1]) + s32[:, 2] * s32[:, 2]), f32(1e-12))[:, None]
+    return n.astype(f32)
+
+
+STITCHED_FORMS = ("seams", "permuted", "flat")
+
+
+def stitched_icosphere(form: str, frequency: int = 8, seed: int = 0):
+    """icosphere_mesh(frequency) with one cell_atlas_uv corner per face corner (v_tex [3F,2], t_tex_idx = arange),
+    in one of three forms of the (v_pos, t_pos_idx) / stitched (v, f) pair that TexturedMesh.set_stitched_mesh takes:
+
+    - "seams": what load_mesh makes of a trimesh asset with merge_vertices=True -- v_pos split per face corner
+      (V = 3F, t_pos_idx = arange, like t_tex_idx), the stitched mesh the merged icosphere (Vn < V);
+    - "permuted": v_pos the merged icosphere, the stitched vertices the same points in a random order (Vn == V) and
+      the stitched faces inv_perm[t_pos_idx]: in range, but not the position indices;
+    - "flat": v_pos merged, the stitched mesh split per face corner (Vn = 3F > V): every normal is a face normal.
+
+    Returns dict(v_pos, t_pos_idx, v_tex, t_tex_idx, stitched_v_pos, stitched_t_pos_idx) as float32 / int32."""
+    from worldrenderer_b200 import synth
+    v, f = icosphere_mesh(frequency)
+    F = f.shape[0]
+    corners = np.arange(3 * F, dtype=np.int32).reshape(-1, 3)
+    vt, ft = synth.cell_atlas_uv(F)
+    if form == "seams":
+        v_pos, t_pos, sv, sf = v[f.reshape(-1)], corners, v, f
+    elif form == "permuted":
+        perm = np.random.default_rng(seed).permutation(v.shape[0])
+        inv = np.argsort(perm).astype(np.int32)
+        v_pos, t_pos, sv, sf = v, f, v[perm], inv[f]
+    elif form == "flat":
+        v_pos, t_pos, sv, sf = v, f, v[f.reshape(-1)], corners
+    else:
+        raise ValueError(form)
+    return dict(v_pos=np.ascontiguousarray(v_pos, f32), t_pos_idx=np.ascontiguousarray(t_pos, np.int32),
+                v_tex=vt.astype(f32), t_tex_idx=ft.astype(np.int32),
+                stitched_v_pos=np.ascontiguousarray(sv, f32), stitched_t_pos_idx=np.ascontiguousarray(sf, np.int32))
+
+
 def terrain_mesh(nx: int = 64, ny: int = 32, seed: int = 0):
     from worldrenderer_b200 import synth
     v, f = synth.terrain(nx, ny, seed)

@@ -157,17 +157,7 @@ def test_vertex_normals_are_exact_sums_independent_of_order(wr_ctx):
     c = make_mesh(v, f[perm], dev).v_nrm
     assert torch.equal(a, b) and torch.equal(a, c)
     # against the exact sum in float64
-    vv, ff = v.astype(np.float64), f.astype(np.int64)
-    e1 = (v[ff[:, 1]] - v[ff[:, 0]]).astype(np.float32)
-    e2 = (v[ff[:, 2]] - v[ff[:, 0]]).astype(np.float32)
-    fn = np.stack([e1[:, 1] * e2[:, 2] - e1[:, 2] * e2[:, 1], e1[:, 2] * e2[:, 0] - e1[:, 0] * e2[:, 2],
-                   e1[:, 0] * e2[:, 1] - e1[:, 1] * e2[:, 0]], -1).astype(np.float32)   # float face normals, as on the GPU
-    acc = np.zeros((v.shape[0], 3), np.float64)
-    for k in range(3):
-        np.add.at(acc, ff[:, k], fn.astype(np.float64))
-    s32 = acc.astype(np.float32)
-    n = s32 / np.maximum(np.sqrt((s32[:, 0] * s32[:, 0] + s32[:, 1] * s32[:, 1]) + s32[:, 2] * s32[:, 2]), np.float32(1e-12))[:, None]
-    np.testing.assert_allclose(a.cpu().numpy(), n.astype(np.float32), rtol=0, atol=1.2e-7)
+    np.testing.assert_allclose(a.cpu().numpy(), cases.exact_vertex_normals(v, f), rtol=0, atol=1.2e-7)
 
 
 def test_single_view_indexing_and_no_cpu_path(wr_ctx):
