@@ -5,8 +5,8 @@ The path keeps 8-byte compact records per (vertex, view) and evaluates one-sampl
 products; everything it cannot represent must fall back to the contract's own classification (cold path) or
 to the queues.  These cases aim at exactly those seams: samples on edges and vertices (fill rule), both
 windings, depth ties, vertices behind the camera / beyond near and far / far off screen, large triangles among
-small ones, odd view counts (padded record rows), more views than one compaction chunk, and the prefilled
-shading variant next to the generic one."""
+small ones, odd view counts (padded record rows), more views than one compaction chunk, and the default
+render() shading instantiation next to the generic one."""
 import numpy as np
 import pytest
 import torch
@@ -40,7 +40,7 @@ def _cam(mvp, dev):
 
 def _check(ctx, mesh, cam, H, W, atol=1e-6):
     """ids / mask / rast bit-exact through the generic shading instantiation, then the default render()
-    (prefilled instantiation) against the oracle's maps."""
+    (k_shade<kOutsRenderDefault, ·>) against the oracle's maps."""
     v = mesh.v_pos.cpu().numpy()
     f = mesh.t_pos_idx.cpu().numpy().astype(np.int32)
     ref = render_oracle.render(v, f, cam.mvp_mtx.cpu().numpy(), cam.w2c.cpu().numpy(), H, W,

@@ -1,5 +1,4 @@
-"""Coarse meshes (few large triangles): set-up / queue-pass times of render() and uv_precompute at large atlases.
-Run with WR_B200_LIB pointing at a -DWR_TILES=0 build for the stripe pass (tools/variants.py)."""
+"""Coarse meshes (few large triangles): set-up / queue-pass times of render() and uv_precompute at large atlases."""
 import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__))); sys.path.insert(0, ROOT)

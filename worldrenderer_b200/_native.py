@@ -13,8 +13,8 @@ from typing import Optional
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# WR_B200_LIB: measurement aid only (tools/variants.py builds the same sources with different -D switches and
-# times them side by side); it must still point at a build of this library -- there is no other implementation.
+# WR_B200_LIB: measurement aid only (time two builds of this library side by side, e.g. before and after a change);
+# it must still point at a build of this library -- there is no other implementation.
 LIB_PATH = os.environ.get("WR_B200_LIB") or os.path.join(_HERE, "lib", "libwr_b200.so")
 
 _c_f32p = ctypes.c_void_p

@@ -644,10 +644,7 @@ extern "C" int wr_view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mas
     const int lead = (hd + 3) & ~3;
     const int boxw = (lead + kPrepTW + hd + 3) & ~3, boxh = kPrepTH + 2 * hd;
     int use_tma = 0;
-#ifndef WR_PREP_TMA
-#define WR_PREP_TMA 1
-#endif
-    if (WR_PREP_TMA && dilation > 0 && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(depth) & 15u) == 0 && boxw <= 256 && boxh <= 256) {
+    if (dilation > 0 && (W & 3) == 0 && (reinterpret_cast<uintptr_t>(depth) & 15u) == 0 && boxw <= 256 && boxh <= 256) {
         static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
         static bool looked_up = false;
         if (!looked_up) {

@@ -23,10 +23,7 @@ constexpr int kPbHalo = 8;                      // sweeps per launch = halo widt
 constexpr int kPbRegW = 128, kPbRegH = 64;      // region held by one block (32 x 64 / kPbRows threads)
 constexpr int kPbOutW = kPbRegW - 2 * kPbHalo;  // 112
 constexpr int kPbOutH = kPbRegH - 2 * kPbHalo;  // 48
-#ifndef WR_PB_ROWS
-#define WR_PB_ROWS 8
-#endif
-constexpr int kPbRows = WR_PB_ROWS;             // region rows per thread (4 columns wide)
+constexpr int kPbRows = 8;                      // region rows per thread (4 columns wide)
 
 struct PbPlanes {
     int H, W, C;

@@ -217,11 +217,10 @@ __device__ __forceinline__ void setup_one(const RasterParams &P, const SnapVert 
 }
 
 template <int LPT>
-__global__ void __launch_bounds__(256) k_setup_triangles(RasterParams P, int view0, const __grid_constant__ FillJob fill)
+__global__ void __launch_bounds__(256) k_setup_triangles(RasterParams P, int view0)
 {
     wr_pdl_wait();
     wr_pdl_trigger();
-    wr_fill_share(fill, blockIdx.y * gridDim.x + blockIdx.x);
     const int gt = blockIdx.x * blockDim.x + threadIdx.x;
     const int t = gt / LPT;
     const int sub = gt % LPT;
@@ -618,16 +617,11 @@ __device__ __forceinline__ void mv_cold(const RasterParams &Pold, const VtxSrc &
     setup_one<1>(Pold, a, c, d, t, 0, depth_view, push, entry, b);
 }
 
-#ifndef WR_MV_MINB
-#define WR_MV_MINB 8
-#endif
 // One thread per (view, triangle), blockIdx.y = view: the parallelism of k_setup_triangles with the compact records.
-__global__ void __launch_bounds__(256, WR_MV_MINB) k_setup_mv(MvParams P, RasterParams Pold, VtxSrc src,
-                                                              const __grid_constant__ FillJob fill)
+__global__ void __launch_bounds__(256, 8) k_setup_mv(MvParams P, RasterParams Pold, VtxSrc src)
 {
     wr_pdl_wait();
     wr_pdl_trigger();
-    wr_fill_share(fill, blockIdx.y * gridDim.x + blockIdx.x);
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int b = blockIdx.y;
     int push = 0;
@@ -1086,15 +1080,7 @@ __device__ __forceinline__ void raster_tiles(const RasterParams &P, const VtxSrc
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
                         const int ry = r0 + ly + j;
-#ifdef WR_TILE_PLAIN
-                        if (ry <= r1 && best[j] != WR_EMPTY_PIXEL) {
-                            unsigned long long *q = depth_view + ((size_t)ry * W + cx);
-                            const unsigned long long cur = *q;
-                            if (best[j] < cur) *q = best[j];
-                        }
-#else
                         if (ry <= r1 && best[j] != WR_EMPTY_PIXEL) atomicMin(depth_view + ((size_t)ry * W + cx), best[j]);
-#endif
                     }
                 }
             }
@@ -1112,14 +1098,11 @@ __global__ void __launch_bounds__(256, 3) k_raster_queues(RasterParams P, VtxSrc
     wr_pdl_trigger();
     const int b = blockIdx.y + view0;
     raster_queue<false>(P, src, b, clip_smem);
-    // large triangles: the tile pass when the view queued few enough of them (WR_TILES=0 keeps the stripe pass)
-#ifndef WR_TILES
-#define WR_TILES 1
-#endif
-    // The tile pass pays off when the large triangles are large against a tile (measured, tools/exp_big.py: from
-    // ~128 tiles of pixel bounding box per triangle on average); below that the stripe pass' parallelism wins.
+    // Large triangles: the tile pass when the view queued few enough of them and they are large against a tile
+    // (measured, tools/exp_big.py: from ~128 tiles of pixel bounding box per triangle on average); below that the
+    // stripe pass' parallelism wins.
     const int nlarge = P.counters[4 * b + 1];
-    const bool tiles = WR_TILES && nlarge > 0 && nlarge <= kTileMaxQueue &&
+    const bool tiles = nlarge > 0 && nlarge <= kTileMaxQueue &&
                        (long long)P.counters[4 * b + 2] >= (long long)kTileMinAvgTiles * nlarge;
     raster_queue<true>(P, src, b, clip_smem, tiles);
     if (tiles) raster_tiles(P, src, b, nlarge, tile_smem);
@@ -1171,18 +1154,12 @@ __global__ void __launch_bounds__(256) k_resolve_rast(unsigned long long *packed
 // scratch are reserved behind the raster buffers and returned through `extra`.
 int wr_run_raster(wr_ctx *ctx, const VtxSrc &src, int B, const int32_t *tri, int F, const int32_t *tri_ranges,
                   int H, int W, size_t extra_bytes, RasterResult *res, void **extra, cudaStream_t stream,
-                  VertexPack *pack, const FillJob *fill)
+                  VertexPack *pack)
 {
-    FillJob no_fill;
-    no_fill.nseg = 0; no_fill.total16 = 0; no_fill.stride = 1; no_fill.shares = 1;
-    FillJob FJ = fill ? *fill : no_fill;
     const int V = src.V;
     // Multi-view fast path (k_snap_mv / k_setup_mv): fused render of a mesh whose triangles are small for this
     // viewport.  Coarse meshes keep the per-view kernels with several lanes per triangle.
-#ifndef WR_MV
-#define WR_MV 1
-#endif
-    const bool use_mv = WR_MV && src.mvp && !tri_ranges && W <= 2048 && H <= 2048 && F > 0 && V > 0 &&
+    const bool use_mv = src.mvp && !tri_ranges && W <= 2048 && H <= 2048 && F > 0 && V > 0 &&
                         (long long)F * 4 > (long long)H * W && (long long)V * B < (1ll << 31);
     const size_t sv_bytes = use_mv ? wr_align256((size_t)V * B * sizeof(int2))
                                    : wr_align256((size_t)B * (size_t)(V > 0 ? V : 1) * sizeof(SnapVert));
@@ -1225,7 +1202,6 @@ int wr_run_raster(wr_ctx *ctx, const VtxSrc &src, int B, const int32_t *tri, int
     res->packed = depth;
     res->packed_bytes = packed_bytes;
     res->view_stats = stats + 4 * B;
-    res->filled = (have_work && !tri_ranges && FJ.nseg > 0) ? 1 : 0;
 
     if (have_work) {
         RasterParams P;
@@ -1253,8 +1229,7 @@ int wr_run_raster(wr_ctx *ctx, const VtxSrc &src, int B, const int32_t *tri, int
             WR_CHECK_LAUNCH(ctx, "k_snap_mv");
             wr_stage(ctx, stream, "k_setup_triangles");
             const bool pdl = !ctx->profiling;
-            wr_fill_plan(&FJ, (unsigned)(wr_div_up(F, 256) * B));
-            wr_launch(k_setup_mv, dim3(wr_div_up(F, 256), B), dim3(256), stream, pdl, M, P, src, FJ);
+            wr_launch(k_setup_mv, dim3(wr_div_up(F, 256), B), dim3(256), stream, pdl, M, P, src);
             WR_CHECK_LAUNCH(ctx, "k_setup_mv");
             wr_stage(ctx, stream, "k_raster_queues");
             wr_launch(k_raster_queues, dim3(qgrid, B), dim3(256), stream, pdl, P, src, 0);
@@ -1270,20 +1245,15 @@ int wr_run_raster(wr_ctx *ctx, const VtxSrc &src, int B, const int32_t *tri, int
         if (!tri_ranges) {
             wr_stage(ctx, stream, "k_setup_triangles");
             const bool pdl = !ctx->profiling && src.mvp != nullptr;  // the chain starts at k_snap_vertices_allviews
-            // coarse mesh for this viewport (expected bounding box of a triangle above ~8 samples): 4 lanes per triangle
-#ifndef WR_SETUP_LPT4
-#define WR_SETUP_LPT4 1
-#endif
-#ifndef WR_SETUP_LPT
-#define WR_SETUP_LPT 4
-#endif
-            const bool lpt4 = WR_SETUP_LPT4 && (long long)F * 4 <= (long long)H * W;
-            wr_fill_plan(&FJ, (unsigned)(wr_div_up((long long)F * (lpt4 ? WR_SETUP_LPT : 1), 256) * B));
+            // coarse mesh for this viewport (expected bounding box of a triangle above ~8 samples): several lanes per
+            // triangle.  2 / 4 / 8 lanes measured 38.4 / 36.7 / 41.0 us on config A (profiles/README.md).
+            constexpr int kCoarseLanes = 4;
+            const bool lpt4 = (long long)F * 4 <= (long long)H * W;
             if (lpt4)
-                wr_launch(k_setup_triangles<WR_SETUP_LPT>, dim3(wr_div_up((long long)F * WR_SETUP_LPT, 256), B), dim3(256),
-                          stream, pdl, P, 0, FJ);
+                wr_launch(k_setup_triangles<kCoarseLanes>, dim3(wr_div_up((long long)F * kCoarseLanes, 256), B), dim3(256),
+                          stream, pdl, P, 0);
             else
-                wr_launch(k_setup_triangles<1>, dim3(wr_div_up(F, 256), B), dim3(256), stream, pdl, P, 0, FJ);
+                wr_launch(k_setup_triangles<1>, dim3(wr_div_up(F, 256), B), dim3(256), stream, pdl, P, 0);
             WR_CHECK_LAUNCH(ctx, "k_setup_triangles");
             wr_stage(ctx, stream, "k_raster_queues");
             wr_launch(k_raster_queues, dim3(qgrid, B), dim3(256), stream, pdl, P, src, 0);
@@ -1295,7 +1265,7 @@ int wr_run_raster(wr_ctx *ctx, const VtxSrc &src, int B, const int32_t *tri, int
                 if (count == 0) continue;
                 RasterParams Q = P;
                 Q.tri = tri + 3 * (size_t)start; Q.F = count; Q.tri_base = start;
-                k_setup_triangles<1><<<dim3(wr_div_up(count, 256), 1), 256, 0, stream>>>(Q, b, no_fill);
+                k_setup_triangles<1><<<dim3(wr_div_up(count, 256), 1), 256, 0, stream>>>(Q, b);
                 WR_CHECK_LAUNCH(ctx, "k_setup_triangles(range)");
                 k_raster_queues<<<dim3(qgrid, 1), 256, 0, stream>>>(Q, src, b);
                 WR_CHECK_LAUNCH(ctx, "k_raster_queues(range)");

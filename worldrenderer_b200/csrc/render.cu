@@ -37,7 +37,6 @@ struct ShadeParams {
     int wide_ok;                 // W % 4 == 0 and 16-byte aligned pos / normal maps: background rows may use 16-byte stores
     int bg_final;                // two-pass depth whose background value is a constant (controlnet, zero123++):
                                  // written here, k_depth_finalize then only touches covered pixels
-    unsigned perm_mul;           // multiplier of the block permutation (0 = identity)
 };
 
 struct PixelGeo {
@@ -210,16 +209,9 @@ __device__ __forceinline__ void shade_covered(const wr_render_args &A, const Tri
     }
 }
 
-#ifndef WR_SHADE_ROWS
-#define WR_SHADE_ROWS 4
-#endif
-#ifndef WR_SHADE_MINB
-#define WR_SHADE_MINB 8   // 64 registers: measured 47.3 us vs 49.6 us unconstrained on config B
-#endif
-#ifndef WR_SHADE_THREADS
-#define WR_SHADE_THREADS 128
-#endif
-constexpr int kShadeRows = WR_SHADE_ROWS;  // rows per thread: that many independent id loads in flight before any use
+constexpr int kShadeRows = 4;       // rows per thread: that many independent id loads in flight before any use
+constexpr int kShadeThreads = 128;
+constexpr int kShadeMinBlocks = 8;  // 64 registers: measured 47.3 us vs 49.6 us unconstrained on config B
 
 // Output sets with their own instantiation (no per-pixel pointer tests, ~30% fewer issued instructions on
 // config B); every other combination runs the generic instantiation (OUTS < 0, runtime tests).
@@ -229,9 +221,8 @@ constexpr int kOutsSimpleDepth = kOutNormal | kOutDepth;                  // mas
 constexpr int kOutsBakeView = kOutGeo | kOutDepth;                        // mask + (pos, aoi_cos) + simple depth
 
 // One column strip of kShadeRows pixels per thread.  grid = (ceil(W/128), ceil(H/kShadeRows), B), 128 threads.
-// PRE: the background of every output has been written by the set-up pass (FillJob): covered pixels only.
-template <int OUTS, bool PACKED, bool PRE>
-__global__ void __launch_bounds__(WR_SHADE_THREADS, WR_SHADE_MINB) k_shade(ShadeParams P)
+template <int OUTS, bool PACKED>
+__global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeParams P)
 {
     const wr_render_args &A = P.a;
     constexpr bool kGeneric = OUTS < 0;
@@ -249,24 +240,11 @@ __global__ void __launch_bounds__(WR_SHADE_THREADS, WR_SHADE_MINB) k_shade(Shade
 
     wr_pdl_wait();
     wr_pdl_trigger();
-    // Block -> strip assignment.  Blocks are dispatched in index order, so with the identity map the blocks resident
-    // at any moment are neighbours in one view: all background (bound by their stores) or all covered (bound by the
-    // latency of their dependent gathers), one phase after the other.  A multiplicative permutation of the linear
-    // block index (P.perm_mul is coprime to the block count) makes the resident set a sample of the whole job, so
-    // that the store-bound and the latency-bound blocks overlap.
-    unsigned bx = blockIdx.x, by = blockIdx.y, bz = blockIdx.z;
-    if (P.perm_mul) {
-        const unsigned n = gridDim.x * gridDim.y * gridDim.z;
-        const unsigned lin = bx + gridDim.x * (by + gridDim.y * bz);
-        const unsigned q = (unsigned)(((unsigned long long)lin * P.perm_mul) % n);
-        bx = q % gridDim.x;
-        const unsigned t2 = q / gridDim.x;
-        by = t2 % gridDim.y;
-        bz = t2 / gridDim.y;
-    }
-    const int c = bx * blockDim.x + threadIdx.x;
-    const int r0 = by * kShadeRows;
-    const int b = bz;
+    // Blocks map to strips in index order; permuting them so that background and covered blocks are resident
+    // together made no difference (profiles/README.md).
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    const int r0 = blockIdx.y * kShadeRows;
+    const int b = blockIdx.z;
     const int W = A.W, H = A.H;
     const bool live = c < W;
 
@@ -300,23 +278,14 @@ __global__ void __launch_bounds__(WR_SHADE_THREADS, WR_SHADE_MINB) k_shade(Shade
     // Strip without a covered pixel in the whole warp (78% of the warps of config B): every lane writes the same
     // constants, so position and normal rows go out as 24 full 16-byte stores each instead of 2 x 3 strided
     // 4-byte stores per lane.  Only the specialised instantiations take it (their output set is known).
-    const float d_bg0 = -(((wz0 * 0.0f + wz1 * 0.0f) + wz2 * 0.0f) + wz3);  // view depth of a background pixel (p = 0)
-    if (PRE) {
-        bool any = false;
-#pragma unroll
-        for (int k = 0; k < kShadeRows; ++k) any |= idw[k] != 0xFFFFFFFFu;
-        if (__ballot_sync(0xFFFFFFFFu, any) == 0) {
-            if (two_pass && nrows > 0) lo = d_bg0;
-            goto publish;
-        }
-    } else if (!kGeneric && !has_geo && P.wide_ok) {
+    if (!kGeneric && !has_geo && P.wide_ok) {
         bool any = false;
 #pragma unroll
         for (int k = 0; k < kShadeRows; ++k) any |= idw[k] != 0xFFFFFFFFu;
         const unsigned lane = threadIdx.x & 31;
         const int cw = c - (int)lane;  // first column of the warp
         if (__ballot_sync(0xFFFFFFFFu, any) == 0 && cw + 32 <= W) {
-            const float d_bg = -(((wz0 * 0.0f + wz1 * 0.0f) + wz2 * 0.0f) + wz3);
+            const float d_bg = -(((wz0 * 0.0f + wz1 * 0.0f) + wz2 * 0.0f) + wz3);  // view depth of a background pixel (p = 0)
             float4 n4;  // elements 4*lane .. 4*lane+3 of the repeating (nbx, nby, nbz) row
             {
                 const int e = (4 * (int)lane) % 3;
@@ -353,10 +322,6 @@ __global__ void __launch_bounds__(WR_SHADE_THREADS, WR_SHADE_MINB) k_shade(Shade
         for (int j = 0; j + 1 < kShadeRows; ++j) idw[j] = idw[j + 1];  // register rotation: no indexed local array
         idw[kShadeRows - 1] = 0xFFFFFFFFu;
         const bool covered = idk != 0xFFFFFFFFu;
-        if (PRE && !covered) {
-            if (two_pass) lo = fminf(lo, d_bg0);
-            continue;
-        }
         int id = -1;
         PixelGeo g;
         g.px = g.py = g.pz = 0.f;
@@ -536,54 +501,9 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
     const bool use_pack = (long long)A.B * A.H * A.W >= 32ll * ((long long)A.V + (want_nrm ? A.Vn : 0));
     pack.pos4 = nullptr;
     pack.nrm4 = nullptr;
-    // Background prefill by the set-up pass (common.cuh FillJob) for the output sets with their own shading
-    // instantiation, when every background value is a constant known now and the maps are 16-byte tileable.
-    FillJob fill;
-    fill.nseg = 0; fill.total16 = 0; fill.stride = 1; fill.shares = 1;
-#ifndef WR_PREFILL
-#define WR_PREFILL 0
-#endif
-    {
-        const bool extras0 = A.out_tri_id || A.out_rast || A.out_attr || A.out_tangent;
-        const bool bg_const = A.out_depth && (A.depth_mode == WR_DEPTH_SIMPLE || A.depth_mode == WR_DEPTH_CONTROLNET ||
-                                              A.depth_mode == WR_DEPTH_ZERO123PP);
-        const bool plain0 = A.out_mask && A.out_pos && A.out_normal && bg_const && !A.out_geo && !extras0;
-        const bool bake0 = A.out_mask && A.out_geo && A.out_depth && A.depth_mode == WR_DEPTH_SIMPLE && !A.out_pos &&
-                           !A.out_normal && !extras0;
-        auto aligned = [](const void *p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; };
-        auto f2u = [](float f) { uint32_t u; memcpy(&u, &f, 4); return u; };
-        auto add = [&](void *ptr, size_t bytes, const uint32_t *period12) {  // period12: 12 words = 3 x uint4
-            FillSeg &sg = fill.seg[fill.nseg++];
-            sg.ptr = static_cast<uint4 *>(ptr);
-            sg.n16 = (unsigned)(bytes / 16);
-            sg.chunk = 0;
-            for (int k = 0; k < 3; ++k) sg.pat[k] = make_uint4(period12[4 * k], period12[4 * k + 1], period12[4 * k + 2], period12[4 * k + 3]);
-            sg.uniform = 1;
-            for (int k = 4; k < 12; ++k) sg.uniform &= period12[k] == period12[k & 3];
-            fill.total16 += sg.n16;
-        };
-        if (WR_PREFILL && (plain0 || bake0) && (npix & 15) == 0 && npix * 16 / 16 < (1ull << 32) && aligned(A.out_mask) && aligned(A.out_depth) &&
-            aligned(A.out_pos) && aligned(A.out_normal) && aligned(A.out_geo)) {
-            uint32_t w[12];
-            for (int k = 0; k < 12; ++k) w[k] = 0;
-            add(A.out_mask, npix, w);
-            for (int k = 0; k < 12; ++k) w[k] = f2u(A.depth_bg);
-            add(A.out_depth, npix * 4, w);
-            if (plain0) {
-                for (int k = 0; k < 12; ++k) w[k] = 0;
-                add(A.out_pos, npix * 12, w);
-                for (int k = 0; k < 12; ++k) w[k] = f2u(A.normal_bg[k % 3]);
-                add(A.out_normal, npix * 12, w);
-            } else {
-                const float aoi_bg = fminf(fmaxf(A.normal_bg[2], 0.0f), 1.0f);
-                for (int k = 0; k < 12; ++k) w[k] = (k & 3) == 3 ? f2u(aoi_bg) : 0u;
-                add(A.out_geo, npix * 16, w);
-            }
-        }
-    }
     int rc = wr_run_raster(ctx, src, A.B, A.tri, A.F, nullptr, A.H, A.W,
                            mask_bytes + (use_pack ? wr_vertex_pack_bytes(A.V, A.Vn, want_nrm) : 0), &res, &extra,
-                           stream, use_pack ? &pack : nullptr, fill.nseg ? &fill : nullptr);
+                           stream, use_pack ? &pack : nullptr);
     if (rc != WR_OK) return rc;
     if (A.raster_done_event) {
         e = cudaEventRecord(static_cast<cudaEvent_t>(A.raster_done_event), stream);
@@ -602,45 +522,24 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
     P.bg_final = two_pass && (A.depth_mode == WR_DEPTH_CONTROLNET || A.depth_mode == WR_DEPTH_ZERO123PP);
     wr_stage(ctx, stream, "k_shade");
     {
-        const dim3 grid(wr_div_up(A.W, WR_SHADE_THREADS), wr_div_up(A.H, kShadeRows), A.B);
-#ifndef WR_SHADE_PERM
-#define WR_SHADE_PERM 0
-#endif
-        P.perm_mul = 0;
-        if (WR_SHADE_PERM) {
-            const unsigned long long n = (unsigned long long)grid.x * grid.y * grid.z;
-            if (n > 64 && n < (1ull << 31)) {
-                // a multiplier near n / golden ratio, made coprime to n
-                unsigned long long m = (unsigned long long)((double)n * 0.6180339887498949) | 1ull;
-                auto gcd = [](unsigned long long a, unsigned long long b) { while (b) { const unsigned long long t = a % b; a = b; b = t; } return a; };
-                while (gcd(m, n) != 1) m += 2;
-                P.perm_mul = (unsigned)(m % n);
-            }
-        }
+        const dim3 grid(wr_div_up(A.W, kShadeThreads), wr_div_up(A.H, kShadeRows), A.B);
         const bool extras = A.out_tri_id || A.out_rast || A.out_attr || A.out_tangent;
         const bool plain = P.mask && A.out_pos && A.out_normal && A.out_depth && !A.out_geo && !extras;
         const bool bake = P.mask && A.out_geo && A.out_depth && !two_pass && !A.out_pos && !A.out_normal && !extras;
         // dependent launch only when the raster stages were launched (the chain's first kernel is a plain launch)
         const bool pdl = !ctx->profiling && A.F > 0 && A.V > 0;
-        const dim3 block(WR_SHADE_THREADS);
-        const bool pre = res.filled != 0;
-#define WR_SHADE_LAUNCH(OUTS, PK) \
-    do { \
-        if (pre) wr_launch(k_shade<OUTS, PK, true>, grid, block, stream, pdl, P); \
-        else wr_launch(k_shade<OUTS, PK, false>, grid, block, stream, pdl, P); \
-    } while (0)
+        const dim3 block(kShadeThreads);
         if (use_pack) {
-            if (plain && two_pass) WR_SHADE_LAUNCH(kOutsRenderDefault, true);
-            else if (plain) WR_SHADE_LAUNCH(kOutsSimpleDepth, true);
-            else if (bake) WR_SHADE_LAUNCH(kOutsBakeView, true);
-            else wr_launch(k_shade<-1, true, false>, grid, block, stream, pdl, P);
+            if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, true>, grid, block, stream, pdl, P);
+            else if (plain) wr_launch(k_shade<kOutsSimpleDepth, true>, grid, block, stream, pdl, P);
+            else if (bake) wr_launch(k_shade<kOutsBakeView, true>, grid, block, stream, pdl, P);
+            else wr_launch(k_shade<-1, true>, grid, block, stream, pdl, P);
         } else {
-            if (plain && two_pass) WR_SHADE_LAUNCH(kOutsRenderDefault, false);
-            else if (plain) WR_SHADE_LAUNCH(kOutsSimpleDepth, false);
-            else if (bake) WR_SHADE_LAUNCH(kOutsBakeView, false);
-            else wr_launch(k_shade<-1, false, false>, grid, block, stream, pdl, P);
+            if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, false>, grid, block, stream, pdl, P);
+            else if (plain) wr_launch(k_shade<kOutsSimpleDepth, false>, grid, block, stream, pdl, P);
+            else if (bake) wr_launch(k_shade<kOutsBakeView, false>, grid, block, stream, pdl, P);
+            else wr_launch(k_shade<-1, false>, grid, block, stream, pdl, P);
         }
-#undef WR_SHADE_LAUNCH
     }
     WR_CHECK_LAUNCH(ctx, "k_shade");
     wr_raster_consumed(ctx, &res);
