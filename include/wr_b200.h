@@ -34,6 +34,7 @@
  *                                    optional multi-GPU all-reduce of the accumulators)
  *   wr_view_scores                   SmartPainter's view scoring loop smart_paint.py:118-158
  *   wr_poisson_blend                 PoissonBlendingSolver.__call__ blend.py:214-324 (Jacobi kernel blend.py:60-100)
+ *   wr_poisson_band_step             (new) wr_poisson_blend split into row bands across the GPUs of a multi-GPU bake
  *   wr_uv_padding / wr_inpaint_u8    uv_padding uv.py:373-382 -> inpaint_cvc cv_ops.py:11-35 (cvcuda.inpaint)
  *
  * The raster contract (snap, fill rule, depth key, tie break) is DESIGN.md section 3.
@@ -63,7 +64,7 @@ const char *wr_status_string(int status);
 const char *wr_ctx_last_error(const wr_ctx *ctx);
 /* Version of this header's ABI (struct layouts included).  wr_version() returns the value the LIBRARY was built with:
  * a caller compiled against another header must not go on (its argument structs have a different layout). */
-#define WR_B200_ABI_VERSION 102
+#define WR_B200_ABI_VERSION 103
 int wr_version(void);
 
 /* One context per (device, stream in flight).  Not thread-safe, like the reference's contexts. */
@@ -267,6 +268,45 @@ int wr_grid_sample(wr_ctx *ctx, const float *map, int B, int H, int W, int C, co
  */
 int wr_poisson_blend(wr_ctx *ctx, const float *src, const uint8_t *mask, const float *tgt, int H, int W, int C,
                      int num_iters, int grad_mode, float *out, void *stream);
+
+/*
+ * wr_poisson_blend split across `world` ranks by row bands (no reference counterpart).  The solve's 112 x 48 output
+ * tiles are dealt out by tile rows: rank r owns tile rows shard_bounds(ceil(H / 48), world)[r] (parallel.py), so the
+ * first ceil(H / 48) % world bands are one tile row taller and, with fewer tile rows than ranks, the last ranks own
+ * none.  Every rank holds the whole src / mask / tgt.  Each point gets the float operations of wr_poisson_blend in
+ * the same order: every rank's output equals wr_poisson_blend's, bit for bit.
+ *
+ * wr_poisson_band_layout reports the sizes of this rank's planes (0 for an empty band), the number of sweep launches
+ * S = ceil(num_iters / 8) and the image rows [row_lo, row_hi) the rank finishes.  Any output pointer may be NULL.
+ *
+ * wr_poisson_band_step launches one step of the solve on `stream`:
+ *   step 0           setup of the local planes (no peer access);
+ *   step 1 .. S      8 Jacobi sweeps of the band (fewer in the last one); from step 2 on, first the 8 halo rows
+ *                    above and below the band are pulled from the neighbouring ranks' iterate plane written by
+ *                    their previous step (16-byte peer loads);
+ *   step S + 1       finish: the band's rows of the result are stored into every rank's output (peer stores).
+ * The caller puts a device-side barrier across the ranks after every step from 1 to S + 1, and after step 0 when
+ * S == 0: a step may only read what the neighbours wrote before the last barrier, and a rank may read its output
+ * after the barrier behind step S + 1.  No kernel waits on another rank.  A rank whose band is empty launches
+ * nothing but must still join every barrier.
+ */
+typedef struct wr_poisson_band_args {
+    const float *src;               /* [H,W,C] guidance, local */
+    const uint8_t *mask;            /* [H,W] solve region, non-zero = inside (as in wr_poisson_blend), local */
+    const float *tgt;               /* [H,W,C], local */
+    int H, W, C;                    /* C <= 4 */
+    int num_iters, grad_mode;       /* as in wr_poisson_blend */
+    int world, rank;                /* world <= WR_MAX_P2P_RANKS */
+    float *xa[WR_MAX_P2P_RANKS];    /* this process's mappings of rank r's two iterate planes (plane_bytes each, */
+    float *xb[WR_MAX_P2P_RANKS];    /* 16-byte aligned); only the own rank's and the neighbours' are read */
+    float *out[WR_MAX_P2P_RANKS];   /* rank r's output [H,W,C] */
+    float *b;                       /* local right-hand side plane (plane_bytes, 16-byte aligned) */
+    uint8_t *m;                     /* local region plane (mask_bytes, 4-byte aligned) */
+    int step;                       /* 0 .. S + 1 */
+} wr_poisson_band_args;
+int wr_poisson_band_layout(int H, int W, int C, int world, int rank, int num_iters, uint64_t *plane_bytes,
+                           uint64_t *mask_bytes, int *steps, int *row_lo, int *row_hi);
+int wr_poisson_band_step(wr_ctx *ctx, const wr_poisson_band_args *args, void *stream);
 
 /*
  * Seam fill standing in for cvcuda.inpaint(image, mask, radius) (cv_ops.py:32; third-party operator, absent):

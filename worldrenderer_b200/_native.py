@@ -26,7 +26,7 @@ SYMBOLS = [
     "wr_ctx_scratch_bytes", "wr_ctx_profile", "wr_ctx_profile_read", "wr_ctx_profile_stage_name", "wr_rasterize", "wr_interpolate", "wr_texture", "wr_vertex_normals",
     "wr_vertex_tangents", "wr_tangent_space_normals",
     "wr_render", "wr_view_prep", "wr_uv_unproject", "wr_uv_finalize", "wr_grid_sample", "wr_uv_reduce_finalize_p2p",
-    "wr_poisson_blend", "wr_inpaint_u8", "wr_uv_padding", "wr_view_scores",
+    "wr_poisson_blend", "wr_poisson_band_layout", "wr_poisson_band_step", "wr_inpaint_u8", "wr_uv_padding", "wr_view_scores",
 ]
 
 DEPTH_NONE, DEPTH_CONTROLNET, DEPTH_ZERO123PP, DEPTH_SIMPLE = 0, 1, 2, 3
@@ -70,7 +70,7 @@ class UnprojectArgs(ctypes.Structure):
     ]
 
 
-ABI_VERSION = 102   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
+ABI_VERSION = 103   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
 MAX_P2P_RANKS = 16
 
 
@@ -82,6 +82,17 @@ class P2PReduceArgs(ctypes.Structure):
         ("mc_accum", ctypes.c_void_p), ("mc_attr", ctypes.c_void_p), ("mc_valid", ctypes.c_void_p),
         ("max_blocks", ctypes.c_int),
         ("tex_lo", ctypes.c_longlong), ("tex_hi", ctypes.c_longlong),
+    ]
+
+
+class PoissonBandArgs(ctypes.Structure):
+    _fields_ = [
+        ("src", ctypes.c_void_p), ("mask", ctypes.c_void_p), ("tgt", ctypes.c_void_p),
+        ("H", ctypes.c_int), ("W", ctypes.c_int), ("C", ctypes.c_int),
+        ("num_iters", ctypes.c_int), ("grad_mode", ctypes.c_int), ("world", ctypes.c_int), ("rank", ctypes.c_int),
+        ("xa", ctypes.c_void_p * MAX_P2P_RANKS), ("xb", ctypes.c_void_p * MAX_P2P_RANKS),
+        ("out", ctypes.c_void_p * MAX_P2P_RANKS), ("b", ctypes.c_void_p), ("m", ctypes.c_void_p),
+        ("step", ctypes.c_int),
     ]
 
 
@@ -139,6 +150,12 @@ def lib() -> ctypes.CDLL:
     L.wr_grid_sample.argtypes = [vp, vp, ci, ci, ci, ci, vp, ci, ci, vp, vp]
     L.wr_poisson_blend.restype = ci
     L.wr_poisson_blend.argtypes = [vp, vp, vp, vp, ci, ci, ci, ci, ci, vp, vp]
+    L.wr_poisson_band_layout.restype = ci
+    u64p = ctypes.POINTER(ctypes.c_uint64)
+    cip = ctypes.POINTER(ci)
+    L.wr_poisson_band_layout.argtypes = [ci, ci, ci, ci, ci, ci, u64p, u64p, cip, cip, cip]
+    L.wr_poisson_band_step.restype = ci
+    L.wr_poisson_band_step.argtypes = [vp, ctypes.POINTER(PoissonBandArgs), vp]
     L.wr_inpaint_u8.restype = ci
     L.wr_inpaint_u8.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp]
     L.wr_view_scores.restype = ci

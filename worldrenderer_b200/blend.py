@@ -35,8 +35,10 @@ class PoissonBlendingSolver:
         n = int(num_iters)
         return n if self.backend == "torch-native" else n - (n & 1)
 
-    def __call__(self, src: SINGLE_IMAGE_TYPE, mask: SINGLE_IMAGE_TYPE, tgt: SINGLE_IMAGE_TYPE, num_iters: int,
-                 inplace: bool = True, grad_mode: str = "src"):
+    def _inputs(self, src: SINGLE_IMAGE_TYPE, mask: SINGLE_IMAGE_TYPE, tgt: SINGLE_IMAGE_TYPE, inplace: bool,
+                grad_mode: str):
+        """(src, mask as u8, tgt, grad-mode index) in the form the kernels take: [H,W,C] float32 on the device,
+        C <= 4, the mask thresholded as in blend.py:229-232."""
         if grad_mode not in _GRAD_MODES:
             raise ValueError(f"Unknown grad_mode: {grad_mode}")
         dev = self._ctx.device
@@ -47,17 +49,19 @@ class PoissonBlendingSolver:
         if src.shape != tgt.shape or mask.shape[:2] != tgt.shape[:2]:
             raise ValueError(f"src {tuple(src.shape)}, mask {tuple(mask.shape)} and tgt {tuple(tgt.shape)} must agree")
         mask = (mask.mean(-1) > 0.5) if mask.ndim == 3 else (mask > 0.5)  # blend.py:229-232
-        H, W, C = tgt.shape
-        if C > 4:
+        if tgt.shape[2] > 4:
             raise NotImplementedError("PoissonBlendingSolver: more than 4 channels")
-        src_c = src.contiguous()
-        mask_c = mask.contiguous().view(torch.uint8)
         if inplace and not tgt.is_contiguous():
             raise ValueError("inplace=True needs a contiguous target")
-        tgt_c = tgt.contiguous()
+        return src.contiguous(), mask.contiguous().view(torch.uint8), tgt.contiguous(), _GRAD_MODES[grad_mode]
+
+    def __call__(self, src: SINGLE_IMAGE_TYPE, mask: SINGLE_IMAGE_TYPE, tgt: SINGLE_IMAGE_TYPE, num_iters: int,
+                 inplace: bool = True, grad_mode: str = "src"):
+        src_c, mask_c, tgt_c, gm = self._inputs(src, mask, tgt, inplace, grad_mode)
+        H, W, C = tgt_c.shape
         out = tgt_c if inplace else torch.empty_like(tgt_c)
         c = self._ctx
         c.check(_native.lib().wr_poisson_blend(c.handle, _native.ptr(src_c), _native.ptr(mask_c), _native.ptr(tgt_c),
-                                               H, W, C, self._sweeps(num_iters), _GRAD_MODES[grad_mode],
+                                               H, W, C, self._sweeps(num_iters), gm,
                                                _native.ptr(out), c.stream()), "wr_poisson_blend")
         return out

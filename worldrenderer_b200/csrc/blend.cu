@@ -28,6 +28,7 @@ constexpr int kPbRows = 8;                      // region rows per thread (4 col
 struct PbPlanes {
     int H, W, C;
     int Hp, Wp;        // padded plane: kPbHalo zero rows / columns in front, rounded up to whole tiles behind
+    int r0;            // image row of plane row kPbHalo (0, or the first row of a band)
     float *xa, *xb;    // [C,Hp,Wp] iterate (0 outside the solve region), ping-pong
     float *b;          // [C,Hp,Wp] right-hand side
     uint8_t *m;        // [Hp,Wp] solve region (image border removed, blend.py:233-236)
@@ -51,7 +52,7 @@ __global__ void __launch_bounds__(256) k_pb_setup(const float *src, const uint8_
     const int pc = blockIdx.x * blockDim.x + threadIdx.x;
     const int pr = blockIdx.y;
     if (pc >= P.Wp) return;
-    const int r = pr - kPbHalo, c = pc - kPbHalo;
+    const int r = pr + P.r0 - kPbHalo, c = pc - kPbHalo;
     const size_t po = (size_t)pr * P.Wp + pc;
     const size_t plane = (size_t)P.Hp * P.Wp;
     const bool inside = r >= 0 && r < P.H && c >= 0 && c < P.W;
@@ -190,13 +191,20 @@ __global__ void __launch_bounds__(32 * (kPbRegH / R), 2) k_pb_jacobi(const float
     }
 }
 
-// out = tgt outside the region, clamp(X, 0, 1) inside (blend.py:317-321)
-__global__ void __launch_bounds__(256) k_pb_finish(const float *tgt, PbPlanes P, const float *x, float *out)
+// Output atlases of k_pb_finish: one, or every rank's (peer stores: the finish of a band solve is its all-gather)
+struct PbOut {
+    float *p[WR_MAX_P2P_RANKS];
+    int n;
+};
+
+// out = tgt outside the region, clamp(X, 0, 1) inside (blend.py:317-321); one thread per pixel of plane row
+// blockIdx.y + kPbHalo, image row blockIdx.y + P.r0
+__global__ void __launch_bounds__(256) k_pb_finish(const float *tgt, PbPlanes P, const float *x, PbOut out)
 {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
-    const int r = blockIdx.y;
+    const int r = blockIdx.y + P.r0;
     if (c >= P.W) return;
-    const size_t po = (size_t)(r + kPbHalo) * P.Wp + (c + kPbHalo);
+    const size_t po = (size_t)(blockIdx.y + kPbHalo) * P.Wp + (c + kPbHalo);
     const size_t plane = (size_t)P.Hp * P.Wp;
     const bool m = P.m[po] != 0;
     const size_t o = ((size_t)r * P.W + c) * P.C;
@@ -208,8 +216,39 @@ __global__ void __launch_bounds__(256) k_pb_finish(const float *tgt, PbPlanes P,
         } else {
             v = __ldg(tgt + o + ch);
         }
-        out[o + ch] = v;
+        for (int k = 0; k < out.n; ++k) out.p[k][o + ch] = v;
     }
+}
+
+// The 2 * kPbHalo halo rows of a band's iterate plane x (kPbHalo above its first tile row, kPbHalo below its last),
+// all channels, pulled with 16-byte loads from the same plane of the neighbouring bands: the last kPbHalo rows the
+// band above owns and the first kPbHalo rows the band below owns.  up / dn are NULL at the edges of the image (the
+// rows there are zero padding, written once by k_pb_setup).  Runs between two sweep launches, after a barrier
+// behind the neighbours' previous launch.
+__global__ void __launch_bounds__(256) k_pb_halo(float *x, int Hp, int Wp, const float *up, int up_Hp, const float *dn,
+                                                 int dn_Hp)
+{
+    wr_pdl_trigger();  // the sweep launch behind may load its region mask and right-hand side meanwhile
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;  // float4 of the row
+    const int i = blockIdx.y;                             // halo row, 0 .. 2 * kPbHalo - 1
+    const bool top = i < kPbHalo;
+    const float *nb = top ? up : dn;
+    if (4 * q >= Wp || !nb) return;
+    const int sr = top ? up_Hp - 2 * kPbHalo + i : i;     // row in the neighbour's plane
+    const int dr = top ? i : Hp - 2 * kPbHalo + i;        // row in this band's plane
+    const size_t nplane = (size_t)(top ? up_Hp : dn_Hp) * Wp;
+    const size_t plane = (size_t)Hp * Wp;
+    const float4 v = *(reinterpret_cast<const float4 *>(nb + blockIdx.z * nplane + (size_t)sr * Wp) + q);
+    *(reinterpret_cast<float4 *>(x + blockIdx.z * plane + (size_t)dr * Wp) + q) = v;
+}
+
+// Tile rows [t0, t1) of the band of `rank`: shard_bounds(tiles_y, world)[rank] of parallel.py (the first
+// tiles_y % world bands one tile row taller).  Non-empty bands are ranks 0 .. min(tiles_y, world) - 1.
+void pb_band(int tiles_y, int world, int rank, int *t0, int *t1)
+{
+    const int base = tiles_y / world, extra = tiles_y % world;
+    *t0 = rank * base + (rank < extra ? rank : extra);
+    *t1 = *t0 + base + (rank < extra ? 1 : 0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -369,7 +408,7 @@ extern "C" int wr_poisson_blend(wr_ctx *ctx, const float *src, const uint8_t *ma
     cudaError_t e = cudaSetDevice(ctx->device);
     if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
     PbPlanes P;
-    P.H = H; P.W = W; P.C = C;
+    P.H = H; P.W = W; P.C = C; P.r0 = 0;
     const int tiles_x = wr_div_up(W, kPbOutW), tiles_y = wr_div_up(H, kPbOutH);
     P.Wp = tiles_x * kPbOutW + 2 * kPbHalo;
     P.Hp = tiles_y * kPbOutH + 2 * kPbHalo;
@@ -399,8 +438,111 @@ extern "C" int wr_poisson_blend(wr_ctx *ctx, const float *src, const uint8_t *ma
         float *t = xin; xin = xout; xout = t;
     }
     wr_stage(ctx, stream, "k_pb_finish");
-    k_pb_finish<<<dim3(wr_div_up(W, 256), H), 256, 0, stream>>>(tgt, P, xin, out);
+    PbOut po = {};
+    po.p[0] = out;
+    po.n = 1;
+    k_pb_finish<<<dim3(wr_div_up(W, 256), H), 256, 0, stream>>>(tgt, P, xin, po);
     WR_CHECK_LAUNCH(ctx, "k_pb_finish");
+    wr_stage(ctx, stream, "end");
+    return WR_OK;
+}
+
+extern "C" int wr_poisson_band_layout(int H, int W, int C, int world, int rank, int num_iters, uint64_t *plane_bytes,
+                                      uint64_t *mask_bytes, int *steps, int *row_lo, int *row_hi)
+{
+    if (H <= 0 || W <= 0 || C <= 0 || C > 4 || world < 1 || world > WR_MAX_P2P_RANKS || rank < 0 || rank >= world ||
+        num_iters < 0)
+        return WR_ERR_INVALID_ARGUMENT;
+    if (H > 16384 || W > 16384) return WR_ERR_UNSUPPORTED;
+    int t0, t1;
+    pb_band(wr_div_up(H, kPbOutH), world, rank, &t0, &t1);
+    const uint64_t Hb = t1 > t0 ? (uint64_t)(t1 - t0) * kPbOutH + 2 * kPbHalo : 0;
+    const uint64_t Wp = (uint64_t)wr_div_up(W, kPbOutW) * kPbOutW + 2 * kPbHalo;
+    if (plane_bytes) *plane_bytes = Hb * Wp * sizeof(float) * C;
+    if (mask_bytes) *mask_bytes = Hb * Wp;
+    if (steps) *steps = wr_div_up(num_iters, kPbHalo);
+    if (row_lo) *row_lo = t0 * kPbOutH < H ? t0 * kPbOutH : H;
+    if (row_hi) *row_hi = t1 * kPbOutH < H ? t1 * kPbOutH : H;
+    return WR_OK;
+}
+
+extern "C" int wr_poisson_band_step(wr_ctx *ctx, const wr_poisson_band_args *args, void *stream_)
+{
+    if (!ctx || !args) return WR_ERR_INVALID_ARGUMENT;
+    const wr_poisson_band_args &A = *args;
+    if (A.H <= 0 || A.W <= 0 || A.C <= 0 || A.C > 4 || A.num_iters < 0 || A.grad_mode < 0 || A.grad_mode > 2 ||
+        A.world < 1 || A.world > WR_MAX_P2P_RANKS || A.rank < 0 || A.rank >= A.world)
+        return WR_ERR_INVALID_ARGUMENT;
+    if (A.H > 16384 || A.W > 16384) return WR_ERR_UNSUPPORTED;
+    const int S = wr_div_up(A.num_iters, kPbHalo);
+    if (A.step < 0 || A.step > S + 1) return WR_ERR_INVALID_ARGUMENT;
+    const int tiles_x = wr_div_up(A.W, kPbOutW), tiles_y = wr_div_up(A.H, kPbOutH);
+    int t0, t1;
+    pb_band(tiles_y, A.world, A.rank, &t0, &t1);
+    if (t1 == t0) return WR_OK;  // no tile row here: this rank only takes part in the barriers
+    // neighbouring bands (empty bands are the last ranks, so they are rank -1 / +1)
+    const int up = t0 > 0 ? A.rank - 1 : -1, dn = t1 < tiles_y ? A.rank + 1 : -1;
+    auto misaligned = [](const void *p, uintptr_t a) { return (reinterpret_cast<uintptr_t>(p) & (a - 1)) != 0; };
+    if (!A.src || !A.mask || !A.tgt || !A.b || !A.m || misaligned(A.b, 16) || misaligned(A.m, 4))
+        return WR_ERR_INVALID_ARGUMENT;
+    for (int r : {A.rank, up, dn}) {
+        if (r < 0) continue;
+        if (!A.xa[r] || !A.xb[r] || misaligned(A.xa[r], 16) || misaligned(A.xb[r], 16)) return WR_ERR_INVALID_ARGUMENT;
+    }
+    for (int r = 0; r < A.world; ++r)
+        if (!A.out[r]) return WR_ERR_INVALID_ARGUMENT;
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    cudaError_t e = cudaSetDevice(ctx->device);
+    if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
+
+    // the band's planes: its tile rows plus kPbHalo rows on either side, the layout of wr_poisson_blend's planes
+    auto band_rows = [&](int r) {
+        int a, b;
+        pb_band(tiles_y, A.world, r, &a, &b);
+        return (b - a) * kPbOutH + 2 * kPbHalo;
+    };
+    PbPlanes P;
+    P.H = A.H; P.W = A.W; P.C = A.C;
+    P.Wp = tiles_x * kPbOutW + 2 * kPbHalo;
+    P.Hp = band_rows(A.rank);
+    P.r0 = t0 * kPbOutH;
+    P.xa = A.xa[A.rank]; P.xb = A.xb[A.rank]; P.b = A.b; P.m = A.m;
+    // launch j (1 .. S) reads plane (j - 1) % 2 and writes plane j % 2 (xa = 0), as in wr_poisson_blend
+    float *const planes[2] = {P.xa, P.xb};
+
+    wr_stage_begin(ctx);
+    if (A.step == 0) {
+        wr_stage(ctx, stream, "k_pb_setup");
+        k_pb_setup<<<dim3(wr_div_up(P.Wp, 256), P.Hp), 256, 0, stream>>>(A.src, A.mask, A.tgt, P, A.grad_mode);
+        WR_CHECK_LAUNCH(ctx, "k_pb_setup");
+    } else if (A.step <= S) {
+        const int par = (A.step - 1) & 1;
+        // launch 1 reads the iterate k_pb_setup wrote on every rank alike: its halo rows are already right
+        const bool halo = A.step > 1 && (up >= 0 || dn >= 0);
+        if (halo) {
+            const float *const *nb = par ? A.xb : A.xa;
+            wr_stage(ctx, stream, "k_pb_halo");
+            k_pb_halo<<<dim3(wr_div_up(P.Wp / 4, 256), 2 * kPbHalo, P.C), 256, 0, stream>>>(
+                planes[par], P.Hp, P.Wp, up >= 0 ? nb[up] : nullptr, up >= 0 ? band_rows(up) : 0,
+                dn >= 0 ? nb[dn] : nullptr, dn >= 0 ? band_rows(dn) : 0);
+            WR_CHECK_LAUNCH(ctx, "k_pb_halo");
+        }
+        const int done = (A.step - 1) * kPbHalo;
+        const int sweeps = A.num_iters - done < kPbHalo ? A.num_iters - done : kPbHalo;
+        wr_stage(ctx, stream, "k_pb_jacobi");
+        wr_launch(k_pb_jacobi<kPbRows>, dim3(tiles_x, t1 - t0, P.C), dim3(32 * (kPbRegH / kPbRows)), stream,
+                  halo && !ctx->profiling, (const float *)planes[par], planes[par ^ 1], (const float *)P.b,
+                  (const uint8_t *)P.m, P.Hp, P.Wp, sweeps);
+        WR_CHECK_LAUNCH(ctx, "k_pb_jacobi");
+    } else {
+        PbOut po = {};
+        for (int r = 0; r < A.world; ++r) po.p[r] = A.out[r];
+        po.n = A.world;
+        const int rows = (t1 * kPbOutH < A.H ? t1 * kPbOutH : A.H) - P.r0;
+        wr_stage(ctx, stream, "k_pb_finish");
+        k_pb_finish<<<dim3(wr_div_up(A.W, 256), rows), 256, 0, stream>>>(A.tgt, P, planes[S & 1], po);
+        WR_CHECK_LAUNCH(ctx, "k_pb_finish");
+    }
     wr_stage(ctx, stream, "end");
     return WR_OK;
 }

@@ -19,7 +19,7 @@ from __future__ import annotations
 import contextlib
 import ctypes
 import warnings
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import torch
 import torch.distributed as dist
@@ -177,23 +177,170 @@ def _p2p_workspace(uv_h: int, uv_w: int, device: torch.device, group, slot: int 
     key = (uv_h, uv_w, device.index, id(group), int(slot))
     ws = _P2P_WORKSPACES.get(key)
     if ws is None:
-        err = None
-        try:
-            ws = P2PBakeWorkspace(uv_h, uv_w, device, group)
-        except Exception as e:
-            ws, err = None, e
-        # symm_mem.empty is a LOCAL allocation: it can fail on one rank only (out of memory).  Agree on the outcome
-        # before anyone commits to a path, or that rank would sit in all_reduce while the others wait on the
-        # symmetric-memory barrier.
-        ok = torch.tensor([0 if ws is None else 1], dtype=torch.int32, device=device)
-        dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=group)
-        if int(ok.item()) == 0:
-            why = f"{type(err).__name__}: {err}" if err is not None else "another rank could not set it up"
-            warnings.warn(f"peer-memory bake unavailable ({why}); using NCCL all_reduce")
+        ws = _agreed_workspace(lambda: P2PBakeWorkspace(uv_h, uv_w, device, group), device, group,
+                               "peer-memory bake unavailable", "using NCCL all_reduce")
+        if ws is None:
             _P2P_DISABLED = True
             return None
         _P2P_WORKSPACES[key] = ws
     return ws
+
+
+def _agreed_workspace(make, device: torch.device, group, what: str, instead: str):
+    """make() on every rank of `group`, or None on every rank if it failed on any (a collective call)."""
+    err = None
+    try:
+        ws = make()
+    except Exception as e:
+        ws, err = None, e
+    # symm_mem.empty is a LOCAL allocation: it can fail on one rank only (out of memory).  Agree on the outcome
+    # before anyone commits to a path, or that rank would sit in all_reduce while the others wait on the
+    # symmetric-memory barrier.
+    ok = torch.tensor([0 if ws is None else 1], dtype=torch.int32, device=device)
+    dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=group)
+    if int(ok.item()) == 0:
+        why = f"{type(err).__name__}: {err}" if err is not None else "another rank could not set it up"
+        warnings.warn(f"{what} ({why}); {instead}")
+        return None
+    return ws
+
+
+class PoissonBandLayout(NamedTuple):
+    plane_bytes: int   # one [C, band rows + 16, padded width] float plane (0: no tile row in this band)
+    mask_bytes: int    # the region plane, one byte per plane point
+    steps: int         # sweep launches S = ceil(num_iters / 8)
+    row_lo: int        # image rows [row_lo, row_hi) this rank finishes
+    row_hi: int
+
+
+def poisson_band_layout(H: int, W: int, C: int, world: int, rank: int, num_iters: int = 0) -> PoissonBandLayout:
+    """Plane sizes and band of `rank` in the banded Poisson solve (wr_poisson_band_layout)."""
+    plane, mask = ctypes.c_uint64(), ctypes.c_uint64()
+    steps, lo, hi = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+    st = _native.lib().wr_poisson_band_layout(H, W, C, world, rank, num_iters, ctypes.byref(plane), ctypes.byref(mask),
+                                              ctypes.byref(steps), ctypes.byref(lo), ctypes.byref(hi))
+    if st != 0:
+        raise ValueError(f"wr_poisson_band_layout({H}, {W}, {C}, world={world}, rank={rank}, num_iters={num_iters}): "
+                         f"{_native.lib().wr_status_string(st).decode()}")
+    return PoissonBandLayout(plane.value, mask.value, steps.value, lo.value, hi.value)
+
+
+def _poisson_band_args(src, mask, tgt, num_iters: int, grad_mode: int, world: int, rank: int, xa, xb, out, b, m):
+    """wr_poisson_band_args of one rank: src / tgt [H,W,C] float32 and mask [H,W] u8 local tensors; xa, xb, out the
+    `world` device addresses of every rank's iterate planes and output atlas; b, m this rank's local planes."""
+    H, W, C = tgt.shape
+    a = _native.PoissonBandArgs()
+    a.src, a.mask, a.tgt = _native.ptr(src), _native.ptr(mask), _native.ptr(tgt)
+    a.H, a.W, a.C, a.num_iters, a.grad_mode, a.world, a.rank = H, W, C, int(num_iters), int(grad_mode), world, rank
+    for r in range(world):
+        a.xa[r], a.xb[r], a.out[r] = xa[r], xb[r], out[r]
+    a.b, a.m = _native.ptr(b), _native.ptr(m)
+    return a
+
+
+def _poisson_band_stages(c: "_native.NativeContext", a: "_native.PoissonBandArgs"):
+    """Launches the steps of one rank's share of a banded Poisson solve on the current stream and yields wherever a
+    barrier across the ranks belongs: after every sweep launch (the next one pulls its halo rows from what the
+    neighbours' launch wrote), before the finish (it stores into every rank's output, which the previous solve's
+    readers may still hold) and after it (every output is complete).  The caller puts the barrier there; every
+    rank yields the same number of times, a rank without a tile row included."""
+    steps = poisson_band_layout(a.H, a.W, a.C, a.world, a.rank, a.num_iters).steps
+    for step in range(steps + 2):
+        a.step = step
+        c.check(_native.lib().wr_poisson_band_step(c.handle, ctypes.byref(a), c.stream()), "wr_poisson_band_step")
+        if step > 0 or steps == 0:
+            yield
+
+
+class PoissonBandWorkspace:
+    """Buffers of the banded Poisson solve of a multi-GPU bake: every rank's two iterate planes and output atlas in
+    torch symmetric memory (the halo rows are pulled from the neighbours' planes and the finished rows stored into
+    every rank's atlas over NVLink / NVSwitch), the right-hand side and region planes local.  Creating one is a
+    collective call."""
+
+    def __init__(self, H: int, W: int, C: int, device: torch.device, group=None):
+        import torch.distributed._symmetric_memory as symm_mem
+        self.group = group if group is not None else dist.group.WORLD
+        self.world, self.rank = dist.get_world_size(self.group), dist.get_rank(self.group)
+        if self.world > _native.MAX_P2P_RANKS:
+            raise RuntimeError(f"at most {_native.MAX_P2P_RANKS} ranks share a banded Poisson solve")
+        self.shape = (H, W, C)
+        lay = [poisson_band_layout(H, W, C, self.world, r) for r in range(self.world)]
+        plane = (max(l.plane_bytes for l in lay) + 255) & ~255   # every rank maps the same symmetric size
+        self._off_xb, self._off_out = plane, 2 * plane
+        self.buf = symm_mem.empty(2 * plane + H * W * C * 4, dtype=torch.uint8, device=device)
+        self.hdl = symm_mem.rendezvous(self.buf, self.group)
+        self.base_ptrs = [int(p) for p in self.hdl.buffer_ptrs]
+        own = lay[self.rank]
+        self.b = torch.empty(own.plane_bytes, dtype=torch.uint8, device=device)
+        self.m = torch.empty(own.mask_bytes, dtype=torch.uint8, device=device)
+        self.out = self.buf[2 * plane:].view(torch.float32).view(H, W, C)
+
+    def barrier(self, channel: int) -> None:
+        self.hdl.barrier(channel=channel)  # device-side, ordered on the current stream
+
+    def solve(self, c: "_native.NativeContext", src, mask, tgt, num_iters: int, grad_mode: int) -> torch.Tensor:
+        """wr_poisson_blend(src, mask, tgt) of the whole atlas on every rank, each rank sweeping its band; the result is
+        `out`, a view of the workspace (valid until the next solve).  Every rank of the group must call it alike."""
+        if tuple(tgt.shape) != self.shape:
+            raise ValueError(f"workspace is for {self.shape}, got {tuple(tgt.shape)}")
+        a = _poisson_band_args(src, mask, tgt, num_iters, grad_mode, self.world, self.rank,
+                               [p for p in self.base_ptrs], [p + self._off_xb for p in self.base_ptrs],
+                               [p + self._off_out for p in self.base_ptrs], self.b, self.m)
+        for _ in _poisson_band_stages(c, a):
+            self.barrier(0)
+        return self.out
+
+
+_PB_WORKSPACES: Dict[tuple, "PoissonBandWorkspace"] = {}
+_PB_DISABLED = False
+
+
+def _poisson_workspace(H: int, W: int, C: int, device: torch.device, group, slot: int = 0) -> Optional[PoissonBandWorkspace]:
+    """Banded-solve workspace `slot` for (atlas size, group), created on first use; None when peer memory is not usable
+    (then every rank runs the whole solve).  A collective call the first time, like _p2p_workspace."""
+    global _PB_DISABLED
+    if _PB_DISABLED or not (dist.is_available() and dist.is_initialized()):
+        return None
+    if dist.get_backend(group) != "nccl" or dist.get_world_size(group) < 2:
+        return None
+    key = (H, W, C, device.index, id(group), int(slot))
+    ws = _PB_WORKSPACES.get(key)
+    if ws is None:
+        ws = _agreed_workspace(lambda: PoissonBandWorkspace(H, W, C, device, group), device, group,
+                               "banded Poisson solve unavailable", "every rank solves the whole atlas")
+        if ws is None:
+            _PB_DISABLED = True
+            return None
+        _PB_WORKSPACES[key] = ws
+    return ws
+
+
+class _BandPoissonSolver:
+    """Stands in for a PoissonBlendingSolver in atlas_postprocess: the same inputs and sweep count, solved by
+    `run(src, mask_u8, tgt, sweeps, grad_mode)` (the banded solve), which returns the blended atlas."""
+
+    def __init__(self, solver, run):
+        self.solver, self.run = solver, run
+
+    def __call__(self, src, mask, tgt, num_iters, inplace=True, grad_mode="src"):
+        assert not inplace   # sharded_bake's tail writes a fresh atlas
+        src_c, mask_c, tgt_c, gm = self.solver._inputs(src, mask, tgt, inplace, grad_mode)
+        return self.run(src_c, mask_c, tgt_c, self.solver._sweeps(num_iters), gm)
+
+
+def _bake_tail(atlas, valid_any, pre, *, uv_padding: bool, poisson_blending: bool, pb_solver, pb_num_iters: int,
+               pb_keep_original_border: bool, from_scratch: bool, band_run=None, native_ctx=None):
+    """The post-processing tail of uv_blend (uv.py:426-461) on the exchanged atlas, on the current stream.  Every
+    padding runs on every rank; with `band_run` (see _BandPoissonSolver) the Poisson solve of a PoissonBlendingSolver
+    is split into row bands across the ranks instead.  Either way the result is identical on every rank."""
+    from .blend import PoissonBlendingSolver
+    from .uv import atlas_postprocess
+    if band_run is not None and poisson_blending and isinstance(pb_solver, PoissonBlendingSolver):
+        pb_solver = _BandPoissonSolver(pb_solver, band_run)
+    return atlas_postprocess(None, atlas, valid_any, pre, do_uv_padding=uv_padding, pad_unseen_area=from_scratch,
+                             poisson_blending=poisson_blending, pb_solver=pb_solver, pb_num_iters=pb_num_iters,
+                             pb_keep_original_border=pb_keep_original_border, native_ctx=native_ctx)
 
 
 _PRE_CACHE: Dict[tuple, tuple] = {}
@@ -224,7 +371,8 @@ def sharded_bake(ctx, mesh, cam_local: Camera, images_local: torch.Tensor, uv_si
                  uv_padding: bool = False, poisson_blending: bool = False, pb_solver=None, pb_num_iters: int = 1000,
                  pb_keep_original_border: bool = True, from_scratch: bool = False, chunks: int = 8,
                  chunk_shape: str = "equal", _slot: int = 0,
-                 _exchange_stream: Optional["torch.cuda.Stream"] = None, _exchange_blocks: int = 0):
+                 _exchange_stream: Optional["torch.cuda.Stream"] = None, _exchange_blocks: int = 0,
+                 _tail_ctx: Optional["_native.NativeContext"] = None):
     """Config E: this rank holds `cam_local` / `images_local` (its share of the views, possibly none);
     the mesh is replicated.  Returns (atlas [uv,uv,3], valid_any [uv,uv] bool), identical on all ranks.
 
@@ -238,15 +386,21 @@ def sharded_bake(ctx, mesh, cam_local: Camera, images_local: torch.Tensor, uv_si
     or "falling" (sizes K : K-1 : ... : 1).
 
     uv_padding / poisson_blending: the post-processing tail of uv_blend (uv.py:426-461) applied to the exchanged
-    atlas.  It is deterministic and cheap next to the exchange, so every rank runs it on its own copy (no second
-    collective); the returned atlas is then a fresh tensor, still identical on all ranks."""
-    from .uv import atlas_postprocess, fused_unproject, fused_view_maps, uv_finalize
+    atlas; the returned atlas is then a fresh tensor, still identical on all ranks.  Every rank runs each seam
+    padding on its own copy.  With peer memory and a PoissonBlendingSolver the Poisson solve is split into row bands,
+    one per rank, that trade 8 halo rows per 8 sweeps and gather the result into every rank's atlas over NVLink; the
+    result is bit-identical to every rank solving the whole atlas, which is what the NCCL path does."""
+    from .blend import PoissonBlendingSolver
+    from .uv import fused_unproject, fused_view_maps, uv_finalize
     if exchange not in ("auto", "p2p", "nccl"):
         raise ValueError(f"exchange={exchange!r}")
     pre = _uv_precompute_cached(ctx, mesh, uv_size)
     ws = _p2p_workspace(uv_size, uv_size, ctx.device, group, _slot) if exchange != "nccl" else None
     if exchange == "p2p" and ws is None:
         raise RuntimeError("exchange='p2p' requested but peer memory is not available for this process group")
+    pws = None
+    if ws is not None and poisson_blending and isinstance(pb_solver, PoissonBlendingSolver):
+        pws = _poisson_workspace(uv_size, uv_size, 3, ctx.device, group, _slot)
     n_local = cam_local.mvp_mtx.shape[0]
     accum = ws.accum if ws is not None else None
     geo = att = None
@@ -291,8 +445,6 @@ def sharded_bake(ctx, mesh, cam_local: Camera, images_local: torch.Tensor, uv_si
                                                       last=k == len(bounds) - 1)
         if xs is None:
             cur.wait_stream(side)
-        if xs is not None:
-            return atlas, valid_any
     else:
         if n_local > 0:
             unproject()
@@ -309,12 +461,18 @@ def sharded_bake(ctx, mesh, cam_local: Camera, images_local: torch.Tensor, uv_si
             else:
                 all_reduce_accumulators(accum, group)
                 atlas, valid_any = uv_finalize(ctx, accum, pre.uv_attr)
-        if xs is not None:
-            return atlas, valid_any
     if uv_padding or poisson_blending:
-        atlas = atlas_postprocess(None, atlas, valid_any, pre, do_uv_padding=uv_padding, pad_unseen_area=from_scratch,
-                                  poisson_blending=poisson_blending, pb_solver=pb_solver, pb_num_iters=pb_num_iters,
-                                  pb_keep_original_border=pb_keep_original_border)
+        if xs is not None:   # BakePipeline: the tail follows the exchange on its stream
+            for t in (pre.uv_mask, pre.uv_attr):
+                if t is not None:
+                    t.record_stream(xs)
+        nctx = _tail_ctx if _tail_ctx is not None else _native.default_context(ctx.device)
+        band_run = (lambda *a: pws.solve(nctx, *a)) if pws is not None else None
+        with torch.cuda.stream(xs) if xs is not None else contextlib.nullcontext():
+            atlas = _bake_tail(atlas, valid_any, pre, uv_padding=uv_padding, poisson_blending=poisson_blending,
+                               pb_solver=pb_solver, pb_num_iters=pb_num_iters,
+                               pb_keep_original_border=pb_keep_original_border, from_scratch=from_scratch,
+                               band_run=band_run, native_ctx=_tail_ctx)
     return atlas, valid_any
 
 
@@ -347,10 +505,14 @@ def _side_stream(device: torch.device) -> "torch.cuda.Stream":
     return s
 
 
+_TAIL_FLAGS = ("uv_padding", "poisson_blending", "pb_solver", "pb_num_iters", "pb_keep_original_border", "from_scratch")
+
+
 class BakeTicket:
-    """Result of one `BakePipeline.submit`: `result()` makes the current stream wait for the exchange and returns
-    (atlas [uv,uv,3], valid_any [uv,uv] bool), identical on every rank.  With peer memory the tensors are views of a
-    pipeline slot: valid until `depth` more bakes have been submitted."""
+    """Result of one `BakePipeline.submit`: `result()` makes the current stream wait for the exchange (and the
+    post-processing tail, if asked for) and returns (atlas [uv,uv,3], valid_any [uv,uv] bool), identical on every
+    rank.  With peer memory the tensors are views of a pipeline slot: valid until `depth` more bakes have been
+    submitted (a post-processed atlas is a fresh tensor)."""
 
     def __init__(self, atlas, valid_any, done: "torch.cuda.Event", device):
         self._atlas, self._valid, self._done, self._device = atlas, valid_any, done, device
@@ -368,9 +530,17 @@ class BakePipeline:
     is), so a single bake cannot scale past compute / (compute + exchange).  A batch can: the exchange of bake k runs
     on its own stream, on pipeline slot k % depth (accumulators, atlas and barrier pads of its own in symmetric
     memory), while the compute stream already renders bake k + 1.  Throughput is then bounded by the longer of the two
-    stages instead of their sum.  Every rank must submit the same bakes in the same order."""
+    stages instead of their sum.  Every rank must submit the same bakes in the same order.
 
-    def __init__(self, ctx, uv_size: int, depth: int = 2, group=None, exchange: str = "auto", exchange_blocks_per_sm: int = 1):
+    postprocess: the post-processing tail every bake of the pipeline gets, as a dict of sharded_bake's tail flags
+    (uv_padding, poisson_blending, pb_solver, pb_num_iters, pb_keep_original_border, from_scratch); None = the
+    exchanged atlas.  The tail runs on the exchange stream behind the exchange of the same bake, with a native context
+    of its own (the compute stream is already rendering the next bake with `ctx`).  With peer memory and a
+    PoissonBlendingSolver the Poisson solve is banded across the ranks, with a workspace per slot set up here.  The
+    tail is fixed per pipeline, not per bake: `submit` refuses these flags."""
+
+    def __init__(self, ctx, uv_size: int, depth: int = 2, group=None, exchange: str = "auto", exchange_blocks_per_sm: int = 1,
+                 postprocess: Optional[dict] = None):
         self.ctx, self.uv_size, self.depth, self.group, self.exchange = ctx, int(uv_size), max(1, int(depth)), group, exchange
         # the exchange kernel with its default grid (8 blocks per SM) takes every thread slot of the GPU and, at
         # high priority, simply runs INSTEAD of the next bake's view passes (measured: no overlap at all); it is bound
@@ -382,14 +552,23 @@ class BakePipeline:
         self._xs = torch.cuda.Stream(self.device, priority=-1)
         self._done: List[Optional[torch.cuda.Event]] = [None] * self.depth
         self._k = 0
+        self._tail = dict(postprocess or {})
+        unknown = set(self._tail) - set(_TAIL_FLAGS)
+        if unknown:
+            raise ValueError(f"postprocess: unknown flags {sorted(unknown)}")
+        self._tail_ctx = _native.NativeContext(self.device) if self._tail else None
         if exchange != "nccl":   # collective set-up of every slot, up front and in the same order on all ranks
+            from .blend import PoissonBlendingSolver
+            banded = self._tail.get("poisson_blending") and isinstance(self._tail.get("pb_solver"), PoissonBlendingSolver)
             for slot in range(self.depth):
-                _p2p_workspace(self.uv_size, self.uv_size, self.device, group, slot)
+                if _p2p_workspace(self.uv_size, self.uv_size, self.device, group, slot) is not None and banded:
+                    _poisson_workspace(self.uv_size, self.uv_size, 3, self.device, group, slot)
 
     def submit(self, mesh, cam_local: Camera, images_local: torch.Tensor, **bake_kwargs) -> BakeTicket:
-        for k in ("uv_padding", "poisson_blending"):
-            if bake_kwargs.get(k):
-                raise NotImplementedError("BakePipeline returns the exchanged atlas; run the post-processing tail on it")
+        for k in _TAIL_FLAGS:
+            if k in bake_kwargs:
+                raise NotImplementedError("BakePipeline runs the post-processing tail given to its constructor "
+                                          "(postprocess=...); it is not chosen per bake")
         slot = self._k % self.depth
         self._k += 1
         cur = torch.cuda.current_stream(self.device)
@@ -397,7 +576,8 @@ class BakePipeline:
             cur.wait_event(self._done[slot])
         atlas, valid_any = sharded_bake(self.ctx, mesh, cam_local, images_local, self.uv_size, group=self.group,
                                         exchange=self.exchange, _slot=slot, _exchange_stream=self._xs,
-                                        _exchange_blocks=self._xblocks, **bake_kwargs)
+                                        _exchange_blocks=self._xblocks, _tail_ctx=self._tail_ctx, **self._tail,
+                                        **bake_kwargs)
         done = torch.cuda.Event()
         done.record(self._xs)
         self._done[slot] = done

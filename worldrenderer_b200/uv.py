@@ -280,10 +280,12 @@ class RandomChoiceBlend(UVBlendWeightStrategy):
         return F.one_hot(w.max(dim=0).indices, num_classes=w.shape[0]).float().permute(2, 0, 1)
 
 
-def uv_padding(attr: torch.Tensor, inside_mask: torch.Tensor, radius: int):
+def uv_padding(attr: torch.Tensor, inside_mask: torch.Tensor, radius: int, native_ctx=None):
     """Seam padding (uv.py:373-382): clamp to [0,1], quantise like inpaint_cvc (cv_ops.py:23-35), fill the
     texels outside `inside_mask`.  One `wr_uv_padding` call (clamp + quantise + fill + /255 fused); the fill is
-    this package's own (cv_ops.py docstring), not cvcuda's."""
+    this package's own (cv_ops.py docstring), not cvcuda's.  native_ctx: the _native.NativeContext whose scratch
+    the call uses (default: the device's shared one); a caller that pads on a second stream while the first one
+    still uses the shared context passes its own."""
     if attr.ndim != 3 or inside_mask.shape != attr.shape[:2]:
         raise ValueError(f"uv_padding: attr [H,W,C] and inside_mask [H,W] expected, got {tuple(attr.shape)}, "
                          f"{tuple(inside_mask.shape)}")
@@ -291,7 +293,7 @@ def uv_padding(attr: torch.Tensor, inside_mask: torch.Tensor, radius: int):
     m = (inside_mask != 0).contiguous().view(torch.uint8)
     H, W, C = a.shape
     out = torch.empty_like(a)
-    c = _native.default_context(a.device)
+    c = native_ctx if native_ctx is not None else _native.default_context(a.device)
     c.check(_native.lib().wr_uv_padding(c.handle, _native.ptr(a), _native.ptr(m), H, W, C, int(radius),
                                         _native.ptr(out), c.stream()), "wr_uv_padding")
     return out
@@ -335,26 +337,27 @@ def uv_blend(
 
 def atlas_postprocess(blend, stitched, valid_any, pre: UVPrecomputeOutput, *, do_uv_padding=True,
                       uv_padding_radius=3, pad_unseen_area=False, poisson_blending=False, pb_solver=None,
-                      pb_num_iters=1000, pb_keep_original_border=True, pb_inplace=False, pb_grad_mode="src"):
+                      pb_num_iters=1000, pb_keep_original_border=True, pb_inplace=False, pb_grad_mode="src",
+                      native_ctx=None):
     """Tail of uv_blend (uv.py:426-461) shared by the step-by-step and the fused bake: optional Poisson blend of
     the projected colours into the existing texture, then seam padding.  `blend` is the weighted view sum,
     `stitched` the same with the existing texture where no view is valid.  Where only texels outside
     `valid_any` differ (they are refilled by the padding before anything reads them) either may stand in for
-    `blend`, which is how the fused bake calls it with blend=None."""
+    `blend`, which is how the fused bake calls it with blend=None.  native_ctx: passed on to `uv_padding`."""
     if poisson_blending:
         assert do_uv_padding  # uv.py:427
         assert pb_solver is not None
-        padded = uv_padding(stitched if blend is None else blend, valid_any, uv_padding_radius)
+        padded = uv_padding(stitched if blend is None else blend, valid_any, uv_padding_radius, native_ctx)
         if pb_keep_original_border:
             pb_tgt = pre.uv_attr
         else:
-            pb_tgt = uv_padding(stitched, pre.uv_mask, uv_padding_radius)
+            pb_tgt = uv_padding(stitched, pre.uv_mask, uv_padding_radius, native_ctx)
         out = pb_solver(padded, valid_any, pb_tgt, pb_num_iters, inplace=pb_inplace, grad_mode=pb_grad_mode)
     else:
         out = stitched
     if do_uv_padding:
         content = valid_any if pad_unseen_area else pre.uv_mask
-        out = uv_padding(out, content, uv_padding_radius)
+        out = uv_padding(out, content, uv_padding_radius, native_ctx)
     return out
 
 
