@@ -24,6 +24,7 @@
  *                                    texture fetch render.py:260-269, normal normalise render.py:275-277
  *   wr_view_prep                     uv_render_geometry view side: camera-space normal + aoi_cos
  *                                    uv.py:108-119, Sobel + max-pool depth gradient uv.py:122-141
+ *   wr_view_prep_sets                (new) the fused bake's view prep for up to four image sets of one rig
  *   wr_uv_unproject                  texel side of uv_render_geometry uv.py:87-90,143-169,
  *                                    uv_render_attr uv.py:193-222, SimpleUVValidityStrategy
  *                                    uv.py:248-298, ExponentialBlend uv.py:317-348, the view sum of
@@ -36,6 +37,7 @@
  *   wr_poisson_blend                 PoissonBlendingSolver.__call__ blend.py:214-324 (Jacobi kernel blend.py:60-100)
  *   wr_poisson_band_step             (new) wr_poisson_blend split into row bands across the GPUs of a multi-GPU bake
  *   wr_uv_padding / wr_inpaint_u8    uv_padding uv.py:373-382 -> inpaint_cvc cv_ops.py:11-35 (cvcuda.inpaint)
+ *   wr_uv_padding_sets               (new) wr_uv_padding of up to four 3-channel atlases against one mask
  *
  * The raster contract (snap, fill rule, depth key, tie break) is DESIGN.md section 3.
  */
@@ -64,7 +66,7 @@ const char *wr_status_string(int status);
 const char *wr_ctx_last_error(const wr_ctx *ctx);
 /* Version of this header's ABI (struct layouts included).  wr_version() returns the value the LIBRARY was built with:
  * a caller compiled against another header must not go on (its argument structs have a different layout). */
-#define WR_B200_ABI_VERSION 103
+#define WR_B200_ABI_VERSION 104
 int wr_version(void);
 
 /* One context per (device, stream in flight).  Not thread-safe, like the reference's contexts. */
@@ -176,6 +178,21 @@ int wr_view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mask, const fl
                  int dilation, float *aoi_cos, float *depth_grad, float *geo_map, float *attr_map,
                  void *stream);
 
+/*
+ * Bake of several image sets of one camera rig in one pass (CameraProjection.project_sets): every set shares the
+ * geometry, the validity and the weights, only the colours differ.
+ */
+#define WR_MAX_BAKE_SETS 4
+
+/*
+ * View prep of the fused bake for K image sets (1 <= K <= WR_MAX_BAKE_SETS); the geometry map comes from wr_render's
+ * out_geo.  images: HOST array of K device pointers, each [B,H,W,3] f32 (read in place, not copied).
+ * attr_map [B,H,W,K,4]: set 0 is (rgb_0, depth_grad) as in wr_view_prep, set k >= 1 is (rgb_k, 0); K = 1 is exactly
+ * wr_view_prep's attr_map.  depth_grad [B,H,W] may be NULL.  The same kernel as wr_view_prep.
+ */
+int wr_view_prep_sets(wr_ctx *ctx, const float *depth, const float *const *images, int K, int B, int H, int W,
+                      int dilation, float *depth_grad, float *attr_map, void *stream);
+
 typedef struct wr_unproject_args {
     const float *uv_pos;      /* [Hu,Wu,3] */
     const uint8_t *uv_mask;   /* [Hu,Wu] */
@@ -183,7 +200,8 @@ typedef struct wr_unproject_args {
     const float *mvp;         /* [Nv,4,4] */
     int Nv, H, W;             /* views and their resolution */
     const float *geo_map;     /* [Nv,H,W,4] from wr_view_prep */
-    const float *attr_map;    /* [Nv,H,W,4] (rgb, depth_grad); NULL => geometry only */
+    const float *attr_map;    /* [Nv,H,W,4] (rgb, depth_grad), or [Nv,H,W,attr_sets,4] from wr_view_prep_sets;
+                                 NULL => geometry only */
     const float *view_masks;  /* [Nv,H,W] f32 or NULL */
     /* SimpleUVValidityStrategy */
     float pos_error_eps, aoi_cos_thresh, mask_thresh, depth_grad_thresh;
@@ -212,6 +230,14 @@ typedef struct wr_unproject_args {
     /* Texel range [tex_lo, tex_hi) of the flattened atlas this call covers; tex_hi == 0 means all of it.  A multi-GPU
        bake unprojects its atlas chunk by chunk so that the exchange of a finished chunk runs under the next one. */
     long long tex_lo, tex_hi;
+    /* Image sets in attr_map (0 or 1: one; at most WR_MAX_BAKE_SETS).  Set 0 is stitched through old_attr / out_attr
+       above, set k >= 1 through old_attr_more[k - 1] (may be NULL) / out_attr_more[k - 1].  Every set gets the
+       validity and weights of set 0 and its own colour sums, in the order of a one-set call: set k's atlas equals a
+       one-set call on set k's images bit for bit.  attr_sets > 1 needs out_attr and out_valid_any and supports
+       neither accum nor the per-view tensors other than uv_aoi_cos / uv_depth_grad (WR_ERR_UNSUPPORTED). */
+    int attr_sets;
+    const float *old_attr_more[WR_MAX_BAKE_SETS - 1];
+    float *out_attr_more[WR_MAX_BAKE_SETS - 1];
 } wr_unproject_args;
 
 int wr_uv_unproject(wr_ctx *ctx, const wr_unproject_args *args, void *stream);
@@ -322,6 +348,12 @@ int wr_inpaint_u8(wr_ctx *ctx, const uint8_t *img, const uint8_t *mask, int H, i
  */
 int wr_uv_padding(wr_ctx *ctx, const float *attr, const uint8_t *inside_mask, int H, int W, int C, int radius,
                   float *out, void *stream);
+/*
+ * wr_uv_padding of K atlases against one mask (1 <= K <= WR_MAX_BAKE_SETS): attr, out are HOST arrays of K device
+ * pointers to [H,W,3] f32.  One jump flood serves all K; out[k] equals wr_uv_padding(attr[k], C = 3) bit for bit.
+ */
+int wr_uv_padding_sets(wr_ctx *ctx, const float *const *attr, const uint8_t *inside_mask, int H, int W, int K,
+                       int radius, float *const *out, void *stream);
 
 /*
  * View scoring of SmartPainter (smart_paint.py:118-158).  attr: [B,H,W,C] f32 (channel 0 = the rendered score map),

@@ -25,8 +25,9 @@ SYMBOLS = [
     "wr_status_string", "wr_ctx_last_error", "wr_version", "wr_ctx_create", "wr_ctx_destroy",
     "wr_ctx_scratch_bytes", "wr_ctx_profile", "wr_ctx_profile_read", "wr_ctx_profile_stage_name", "wr_rasterize", "wr_interpolate", "wr_texture", "wr_vertex_normals",
     "wr_vertex_tangents", "wr_tangent_space_normals",
-    "wr_render", "wr_view_prep", "wr_uv_unproject", "wr_uv_finalize", "wr_grid_sample", "wr_uv_reduce_finalize_p2p",
-    "wr_poisson_blend", "wr_poisson_band_layout", "wr_poisson_band_step", "wr_inpaint_u8", "wr_uv_padding", "wr_view_scores",
+    "wr_render", "wr_view_prep", "wr_view_prep_sets", "wr_uv_unproject", "wr_uv_finalize", "wr_grid_sample", "wr_uv_reduce_finalize_p2p",
+    "wr_poisson_blend", "wr_poisson_band_layout", "wr_poisson_band_step", "wr_inpaint_u8", "wr_uv_padding", "wr_uv_padding_sets",
+    "wr_view_scores",
 ]
 
 DEPTH_NONE, DEPTH_CONTROLNET, DEPTH_ZERO123PP, DEPTH_SIMPLE = 0, 1, 2, 3
@@ -52,6 +53,9 @@ class RenderArgs(ctypes.Structure):
     ]
 
 
+MAX_BAKE_SETS = 4   # WR_MAX_BAKE_SETS
+
+
 class UnprojectArgs(ctypes.Structure):
     _fields_ = [
         ("uv_pos", ctypes.c_void_p), ("uv_mask", ctypes.c_void_p), ("Hu", ctypes.c_int), ("Wu", ctypes.c_int),
@@ -67,10 +71,12 @@ class UnprojectArgs(ctypes.Structure):
         ("uv_mask_proj", ctypes.c_void_p), ("uv_valid", ctypes.c_void_p), ("uv_weight", ctypes.c_void_p),
         ("old_attr", ctypes.c_void_p), ("out_attr", ctypes.c_void_p), ("out_valid_any", ctypes.c_void_p),
         ("tex_lo", ctypes.c_longlong), ("tex_hi", ctypes.c_longlong),
+        ("attr_sets", ctypes.c_int), ("old_attr_more", ctypes.c_void_p * (MAX_BAKE_SETS - 1)),
+        ("out_attr_more", ctypes.c_void_p * (MAX_BAKE_SETS - 1)),
     ]
 
 
-ABI_VERSION = 103   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
+ABI_VERSION = 104   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
 MAX_P2P_RANKS = 16
 
 
@@ -140,6 +146,8 @@ def lib() -> ctypes.CDLL:
     L.wr_render.argtypes = [vp, ctypes.POINTER(RenderArgs), vp]
     L.wr_view_prep.restype = ci
     L.wr_view_prep.argtypes = [vp, vp, vp, vp, vp, vp, vp, ci, ci, ci, ci, vp, vp, vp, vp, vp]
+    L.wr_view_prep_sets.restype = ci
+    L.wr_view_prep_sets.argtypes = [vp, vp, vp, ci, ci, ci, ci, ci, vp, vp, vp]
     L.wr_uv_unproject.restype = ci
     L.wr_uv_unproject.argtypes = [vp, ctypes.POINTER(UnprojectArgs), vp]
     L.wr_uv_finalize.restype = ci
@@ -162,6 +170,8 @@ def lib() -> ctypes.CDLL:
     L.wr_view_scores.argtypes = [vp, vp, ci, vp, ci, ci, ci, ctypes.c_float, ctypes.c_float, ctypes.c_float, vp, vp, vp]
     L.wr_uv_padding.restype = ci
     L.wr_uv_padding.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp]
+    L.wr_uv_padding_sets.restype = ci
+    L.wr_uv_padding_sets.argtypes = [vp, vp, vp, ci, ci, ci, ci, vp, vp]
     if L.wr_version() != ABI_VERSION:   # a stale library: its argument structs differ from the ones declared here
         raise RuntimeError(f"{LIB_PATH} has ABI version {L.wr_version()}, this package expects {ABI_VERSION}: rebuild it "
                            "with `python -m worldrenderer_b200.build_native --force`")
@@ -174,6 +184,11 @@ def ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     if t is None or t.numel() == 0:
         return None
     return t.data_ptr()
+
+
+def ptr_array(tensors) -> ctypes.Array:
+    """HOST array of device pointers (None stays NULL), for the entry points that take one pointer per image set."""
+    return (ctypes.c_void_p * len(tensors))(*[ptr(t) for t in tensors])
 
 
 def stream_ptr(device: torch.device) -> int:

@@ -9,6 +9,11 @@
 //                      4 taps x 2 x 16-byte loads instead of 4 taps x (12 + 4 + 4 + 12) bytes
 //   k_uv_unproject     per texel: project into every view, gather, validity, weight, accumulate
 //   k_uv_finalize      stitch with the existing texture (after the optional all-reduce)
+//
+// k_view_prep and k_uv_unproject are templated on K, the image sets baked together (CameraProjection.project_sets,
+// up to WR_MAX_BAKE_SETS): the attr map holds K float4 per pixel, set 0 = (rgb_0, depth_grad), set k = (rgb_k, 0),
+// and the unprojection computes the geometry, validity and weights once and keeps K colour sums.  K = 1 is the
+// one-set bake.
 #include <cuda.h>           // CUtensorMap and its enums only: the encoder is fetched through cudaGetDriverEntryPoint (no -lcuda)
 #include <cudaTypedefs.h>   // PFN_cuTensorMapEncodeTiled
 
@@ -69,12 +74,19 @@ __device__ __forceinline__ float window_max(const float *p, int n)
     return m;
 }
 
+// the image sets 1 .. K-1 of a K-set bake (set 0 keeps its own parameter)
+struct ExtraSets {
+    const float *p[WR_MAX_BAKE_SETS - 1];
+};
+
+template <int K>
 __global__ void __launch_bounds__(kPrepTW * kPrepBH) k_view_prep(const float *normal, const uint8_t *mask,
                                                                 const float *depth, const float *position,
                                                                 const float *w2c, const float *images, int H, int W,
                                                                 int dilation, float *aoi_out, float *depth_grad,
                                                                 float *geo_map, float *attr_map,
-                                                                const __grid_constant__ CUtensorMap depth_map, int use_tma)
+                                                                const __grid_constant__ CUtensorMap depth_map, int use_tma,
+                                                                ExtraSets more)
 {
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) unsigned long long s_bar;
@@ -166,7 +178,13 @@ __global__ void __launch_bounds__(kPrepTW * kPrepBH) k_view_prep(const float *no
         if (attr_map) {
             float ir = 0.f, ig = 0.f, ib = 0.f;
             if (images) { const float *im = images + 3 * o; ir = __ldg(im); ig = __ldg(im + 1); ib = __ldg(im + 2); }
-            reinterpret_cast<float4 *>(attr_map)[o] = make_float4(ir, ig, ib, dg);
+            float4 *am = reinterpret_cast<float4 *>(attr_map) + o * K;
+            am[0] = make_float4(ir, ig, ib, dg);
+#pragma unroll
+            for (int k = 1; k < K; ++k) {
+                const float *im = more.p[k - 1] + 3 * o;
+                am[k] = make_float4(__ldg(im), __ldg(im + 1), __ldg(im + 2), 0.0f);
+            }
         }
         if (!normal) continue;  // geometry half already produced by wr_render (out_geo)
         const float *n = normal + 3 * o;
@@ -221,13 +239,15 @@ __device__ __forceinline__ void tap4(float4 &acc, const float4 v, float w)
 }
 
 // Taps are added in the order (0,0), (1,0), (0,1), (1,1); a tap outside the map adds nothing (zero padding).
+// S: float4 per pixel (the image sets of a K-set attr map; the sample reads one of them).
+template <int S = 1>
 __device__ __forceinline__ float4 sample4(const float4 *map, const Bilinear &t, int W, int H)
 {
     float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
     if (!t.ok) return acc;
     if (t.x0 >= 0 && t.y0 >= 0 && t.x0 + 1 < W && t.y0 + 1 < H) {  // interior: one base offset, no per-tap tests
-        const float4 *p = map + ((unsigned)t.y0 * (unsigned)W + (unsigned)t.x0);
-        const float4 v00 = __ldg(p), v10 = __ldg(p + 1), v01 = __ldg(p + W), v11 = __ldg(p + W + 1);
+        const float4 *p = map + ((unsigned)t.y0 * (unsigned)W + (unsigned)t.x0) * S;
+        const float4 v00 = __ldg(p), v10 = __ldg(p + S), v01 = __ldg(p + W * S), v11 = __ldg(p + (W + 1) * S);
         tap4(acc, v00, t.w00); tap4(acc, v10, t.w10); tap4(acc, v01, t.w01); tap4(acc, v11, t.w11);
         return acc;
     }
@@ -236,7 +256,7 @@ __device__ __forceinline__ float4 sample4(const float4 *map, const Bilinear &t, 
     const float ws[4] = { t.w00, t.w10, t.w01, t.w11 };
 #pragma unroll
     for (int k = 0; k < 4; ++k)
-        if (xs[k] >= 0 && xs[k] < W && ys[k] >= 0 && ys[k] < H) tap4(acc, __ldg(map + (size_t)ys[k] * W + xs[k]), ws[k]);
+        if (xs[k] >= 0 && xs[k] < W && ys[k] >= 0 && ys[k] < H) tap4(acc, __ldg(map + ((size_t)ys[k] * W + xs[k]) * S), ws[k]);
     return acc;
 }
 
@@ -268,9 +288,11 @@ __device__ __forceinline__ float blend_pow(float w, float e)
 
 // MATERIALISE: 0 = blend only; 1 = any of the reference's per-view tensors; 2 = only uv_aoi_cos / uv_depth_grad, which
 // is what CameraProjection(return_dict=True) asks for (no view-mask tap for invalid texel-views, no pointer tests
-// for the other seven tensors).
-template <int MATERIALISE>
-__global__ void __launch_bounds__(256) k_uv_unproject(wr_unproject_args A)
+// for the other seven tensors).  K: image sets in attr_map (1 = the one-set bake); K > 1 runs with MATERIALISE 0 or 2.
+// The K > 1 instantiations carry a minimum of 3 blocks per SM (at most 85 registers): left to itself ptxas holds
+// them at 64 registers and spills the extra colour sums.
+template <int MATERIALISE, int K>
+__global__ void __launch_bounds__(256, K > 1 ? 3 : 0) k_uv_unproject(wr_unproject_args A)
 {
     constexpr bool materialise = MATERIALISE != 0;
     constexpr bool light = MATERIALISE == 2;
@@ -300,6 +322,9 @@ __global__ void __launch_bounds__(256) k_uv_unproject(wr_unproject_args A)
     if (o >= (A.tex_hi ? A.tex_hi : ntex)) return;
     const bool inside = A.uv_mask[o] != 0;
     float sr = 0.f, sg = 0.f, sb = 0.f, sw = 0.f;
+    float xr[K], xg[K], xb[K];   // colour sums of the sets 1 .. K-1 (index 0 unused)
+#pragma unroll
+    for (int k = 0; k < K; ++k) xr[k] = xg[k] = xb[k] = 0.f;
     int nvalid = 0;
 
     if (inside || materialise) {
@@ -329,8 +354,9 @@ __global__ void __launch_bounds__(256) k_uv_unproject(wr_unproject_args A)
             bool valid = (err < A.pos_error_eps) && (geo.w > A.aoi_cos_thresh) && inside;
             // the colour / depth-gradient taps only matter for a texel that passed the geometry test
             float4 att = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (A.attr_map && (valid || materialise))
-                att = sample4(reinterpret_cast<const float4 *>(A.attr_map) + v * npix, t, A.W, A.H);
+            const bool tapped = A.attr_map && (valid || materialise);
+            const float4 *amap = reinterpret_cast<const float4 *>(A.attr_map) + v * npix * K;
+            if (tapped) att = sample4<K>(amap, t, A.W, A.H);
             if (A.use_depth_grad) valid = valid && (att.w < A.depth_grad_thresh);
             float mp = 0.f;
             if (A.view_masks && (valid || (materialise && !light))) {
@@ -346,6 +372,15 @@ __global__ void __launch_bounds__(256) k_uv_unproject(wr_unproject_args A)
             wgt = blend_pow(wgt, s_expo[v]);
             sw = sw + wgt;
             sr = sr + att.x * wgt; sg = sg + att.y * wgt; sb = sb + att.z * wgt;
+            // Set k >= 1 is tapped only where its weight is non-zero (for the exponents in use: where the texel-view is
+            // valid).  Where a one-set call on set k tapped anyway, it added colour * 0 = +-0, which leaves a sum of
+            // finite colours unchanged: the sums are those of that call, operation for operation.
+#pragma unroll
+            for (int k = 1; k < K; ++k) {
+                float4 ak = make_float4(0.f, 0.f, 0.f, 0.f);
+                if (tapped && wgt != 0.0f) ak = sample4<K>(amap + k, t, A.W, A.H);
+                xr[k] = xr[k] + ak.x * wgt; xg[k] = xg[k] + ak.y * wgt; xb[k] = xb[k] + ak.z * wgt;
+            }
             nvalid += valid ? 1 : 0;
             if (light) {
                 const size_t ov = (size_t)v * ntex + o;
@@ -389,6 +424,16 @@ __global__ void __launch_bounds__(256) k_uv_unproject(wr_unproject_args A)
             A.out_attr[3 * o] = wr_div_zpos(sr, den) * va + o0 * (1.0f - va);
             A.out_attr[3 * o + 1] = wr_div_zpos(sg, den) * va + o1 * (1.0f - va);
             A.out_attr[3 * o + 2] = wr_div_zpos(sb, den) * va + o2 * (1.0f - va);
+        }
+#pragma unroll
+        for (int k = 1; k < K; ++k) {
+            const float *old = A.old_attr_more[k - 1];
+            float *out = A.out_attr_more[k - 1];
+            float o0 = 0.f, o1 = 0.f, o2 = 0.f;
+            if (old) { o0 = old[3 * o]; o1 = old[3 * o + 1]; o2 = old[3 * o + 2]; }
+            out[3 * o] = wr_div_zpos(xr[k], den) * va + o0 * (1.0f - va);
+            out[3 * o + 1] = wr_div_zpos(xg[k], den) * va + o1 * (1.0f - va);
+            out[3 * o + 2] = wr_div_zpos(xb[k], den) * va + o2 * (1.0f - va);
         }
     }
 }
@@ -620,14 +665,20 @@ extern "C" int wr_grid_sample(wr_ctx *ctx, const float *map, int B, int H, int W
     return WR_OK;
 }
 
-extern "C" int wr_view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mask, const float *depth,
-                            const float *position, const float *w2c, const float *images, int B, int H, int W,
-                            int dilation, float *aoi_cos, float *depth_grad, float *geo_map, float *attr_map,
-                            void *stream_)
+// wr_view_prep / wr_view_prep_sets: images holds K pointers (images[0] may be NULL when K == 1)
+static int view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mask, const float *depth, const float *position,
+                     const float *w2c, const float *const *images, int K, int B, int H, int W, int dilation,
+                     float *aoi_cos, float *depth_grad, float *geo_map, float *attr_map, void *stream_)
 {
     if (!ctx || B < 0 || H <= 0 || W <= 0 || dilation < 0) return WR_ERR_INVALID_ARGUMENT;
     if (dilation > 0 && (dilation & 1) == 0) return WR_ERR_UNSUPPORTED;  // even max-pool changes the map size
     if (B == 0) return WR_OK;
+    ExtraSets more = {};
+    for (int k = 1; k < K; ++k) {
+        if (!images[k]) return WR_ERR_INVALID_ARGUMENT;
+        more.p[k - 1] = images[k];
+    }
+    if (K > 1 && (!images[0] || !attr_map)) return WR_ERR_INVALID_ARGUMENT;
     if (normal) {
         if (!mask || !w2c || (geo_map && !position)) return WR_ERR_INVALID_ARGUMENT;
     } else if (aoi_cos || geo_map) {
@@ -675,11 +726,38 @@ extern "C" int wr_view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mas
     const dim3 grid(wr_div_up(W, kPrepTW), wr_div_up(H, kPrepTH), B);
     wr_stage_begin(ctx);
     wr_stage(ctx, stream, "k_view_prep");
-    wr_launch_s(k_view_prep, grid, dim3(kPrepTW, kPrepBH), dilation > 0 ? smem : 0, stream, !ctx->profiling, normal, mask,
-                depth, position, w2c, images, H, W, dilation, aoi_cos, depth_grad, geo_map, attr_map, tmap, use_tma);
+    auto launch = [&](auto kernel) {
+        wr_launch_s(kernel, grid, dim3(kPrepTW, kPrepBH), dilation > 0 ? smem : 0, stream, !ctx->profiling, normal, mask,
+                    depth, position, w2c, images[0], H, W, dilation, aoi_cos, depth_grad, geo_map, attr_map, tmap, use_tma,
+                    more);
+    };
+    switch (K) {
+    case 1: launch(k_view_prep<1>); break;
+    case 2: launch(k_view_prep<2>); break;
+    case 3: launch(k_view_prep<3>); break;
+    default: launch(k_view_prep<4>); break;
+    }
     WR_CHECK_LAUNCH(ctx, "k_view_prep");
     wr_stage(ctx, stream, "end");
     return WR_OK;
+}
+
+extern "C" int wr_view_prep(wr_ctx *ctx, const float *normal, const uint8_t *mask, const float *depth,
+                            const float *position, const float *w2c, const float *images, int B, int H, int W,
+                            int dilation, float *aoi_cos, float *depth_grad, float *geo_map, float *attr_map,
+                            void *stream_)
+{
+    return view_prep(ctx, normal, mask, depth, position, w2c, &images, 1, B, H, W, dilation, aoi_cos, depth_grad,
+                     geo_map, attr_map, stream_);
+}
+
+extern "C" int wr_view_prep_sets(wr_ctx *ctx, const float *depth, const float *const *images, int K, int B, int H,
+                                 int W, int dilation, float *depth_grad, float *attr_map, void *stream_)
+{
+    if (!images || K < 1 || K > WR_MAX_BAKE_SETS) return WR_ERR_INVALID_ARGUMENT;
+    if (B > 0 && (!attr_map || !images[0])) return WR_ERR_INVALID_ARGUMENT;
+    return view_prep(ctx, nullptr, nullptr, depth, nullptr, nullptr, images, K, B, H, W, dilation, nullptr, depth_grad,
+                     nullptr, attr_map, stream_);
 }
 
 extern "C" int wr_uv_unproject(wr_ctx *ctx, const wr_unproject_args *args, void *stream_)
@@ -691,6 +769,16 @@ extern "C" int wr_uv_unproject(wr_ctx *ctx, const wr_unproject_args *args, void 
     if (A.use_depth_grad && !A.attr_map) return WR_ERR_INVALID_ARGUMENT;
     const size_t smem = (size_t)A.Nv * 17 * sizeof(float);
     if (smem > 48 * 1024) return WR_ERR_UNSUPPORTED;
+    if (A.attr_sets < 0 || A.attr_sets > WR_MAX_BAKE_SETS) return WR_ERR_INVALID_ARGUMENT;
+    const int K = A.attr_sets > 1 ? A.attr_sets : 1;
+    const bool heavy = A.uv_pos_ndc || A.uv_pos_proj || A.uv_pos_error || A.uv_attr_proj || A.uv_mask_proj || A.uv_valid ||
+                       A.uv_weight;
+    if (K > 1) {   // the fused single-GPU form (and the light per-view planes) only
+        if (A.accum || heavy) return WR_ERR_UNSUPPORTED;
+        if (!A.attr_map || !A.out_attr || !A.out_valid_any) return WR_ERR_INVALID_ARGUMENT;
+        for (int k = 0; k < K - 1; ++k)
+            if (!A.out_attr_more[k]) return WR_ERR_INVALID_ARGUMENT;
+    }
     cudaStream_t stream = static_cast<cudaStream_t>(stream_);
     cudaError_t e = cudaSetDevice(ctx->device);
     if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
@@ -699,13 +787,25 @@ extern "C" int wr_uv_unproject(wr_ctx *ctx, const wr_unproject_args *args, void 
     const long long ntex = (long long)A.Hu * A.Wu;
     wr_stage_begin(ctx);
     wr_stage(ctx, stream, "k_uv_unproject");
-    const bool heavy = A.uv_pos_ndc || A.uv_pos_proj || A.uv_pos_error || A.uv_attr_proj || A.uv_mask_proj || A.uv_valid ||
-                       A.uv_weight;
     if (A.tex_lo < 0 || A.tex_hi < 0 || A.tex_hi > ntex || (A.tex_hi && A.tex_lo >= A.tex_hi)) return WR_ERR_INVALID_ARGUMENT;
     const dim3 grid(wr_div_up((A.tex_hi ? A.tex_hi : ntex) - A.tex_lo, 256)), block(256);
-    if (heavy) wr_launch_s(k_uv_unproject<1>, grid, block, smem, stream, !ctx->profiling, A);
-    else if (materialise) wr_launch_s(k_uv_unproject<2>, grid, block, smem, stream, !ctx->profiling, A);
-    else wr_launch_s(k_uv_unproject<0>, grid, block, smem, stream, !ctx->profiling, A);
+    auto launch = [&](auto kernel) { wr_launch_s(kernel, grid, block, smem, stream, !ctx->profiling, A); };
+    if (heavy) launch(k_uv_unproject<1, 1>);
+    else if (materialise) {
+        switch (K) {
+        case 1: launch(k_uv_unproject<2, 1>); break;
+        case 2: launch(k_uv_unproject<2, 2>); break;
+        case 3: launch(k_uv_unproject<2, 3>); break;
+        default: launch(k_uv_unproject<2, 4>); break;
+        }
+    } else {
+        switch (K) {
+        case 1: launch(k_uv_unproject<0, 1>); break;
+        case 2: launch(k_uv_unproject<0, 2>); break;
+        case 3: launch(k_uv_unproject<0, 3>); break;
+        default: launch(k_uv_unproject<0, 4>); break;
+        }
+    }
     WR_CHECK_LAUNCH(ctx, "k_uv_unproject");
     wr_stage(ctx, stream, "end");
     return WR_OK;

@@ -9,6 +9,7 @@
 //   wr_inpaint         uv_padding -> inpaint_cvc uv.py:373-382, cv_ops.py:11-35: quantisation contract of the
 //                      reference, fill by jump flooding + inverse-square-distance average (the cvcuda operator
 //                      is third-party and absent; see oracle/wr_oracle_blend.c for the statement of the fill).
+//                      wr_uv_padding_sets fills up to four 3-channel atlases from one jump flood.
 //
 // CPU statement of both: oracle/wr_oracle_blend.c (bit-identical results; the library is compiled with
 // -fmad=false and IEEE division).
@@ -349,6 +350,58 @@ __global__ void __launch_bounds__(256) k_inpaint_fill(const T *img, const uint8_
     }
 }
 
+// k_inpaint_fill<float> with C = 3 for up to WR_MAX_BAKE_SETS images against one mask and one seed map: every known
+// neighbour is visited and weighted once for all K images.  Each channel gets the float operations of k_inpaint_fill
+// in the same order, so out[k] is what k_inpaint_fill writes for in[k].
+struct PadSets {
+    const float *in[WR_MAX_BAKE_SETS];
+    float *out[WR_MAX_BAKE_SETS];
+};
+
+template <int K>
+__global__ void __launch_bounds__(256) k_inpaint_fill_sets(PadSets S, const uint8_t *inside, const int *seed, int H,
+                                                           int W, int radius)
+{
+    wr_pdl_wait();
+    const int c = blockIdx.x * blockDim.x + threadIdx.x;
+    const int r = blockIdx.y;
+    if (c >= W) return;
+    const size_t p = (size_t)r * W + c;
+    const int q = seed[p];
+    if (inside[p] != 0 || q == kSeedNone) {
+#pragma unroll
+        for (int k = 0; k < K; ++k)
+            for (int ch = 0; ch < 3; ++ch) Quant<float>::store(S.out[k] + p * 3 + ch, Quant<float>::load(S.in[k] + p * 3 + ch));
+        return;
+    }
+    const int qr = q >> 16, qc = q & 0xFFFF;
+    const float num = (float)(1 + seed_dist2(r, c, q));
+    float acc[K][3], ws = 0.0f;
+#pragma unroll
+    for (int k = 0; k < K; ++k) acc[k][0] = acc[k][1] = acc[k][2] = 0.f;
+    for (int tr = max(qr - radius, 0); tr <= min(qr + radius, H - 1); ++tr)
+        for (int tc = max(qc - radius, 0); tc <= min(qc + radius, W - 1); ++tc) {
+            if ((tr - qr) * (tr - qr) + (tc - qc) * (tc - qc) > radius * radius) continue;
+            const size_t t = (size_t)tr * W + tc;
+            if (__ldg(inside + t) == 0) continue;
+            const int dy = r - tr, dx = c - tc;
+            const float w = num / (float)(1 + dy * dy + dx * dx);
+#pragma unroll
+            for (int k = 0; k < K; ++k)
+#pragma unroll
+                for (int ch = 0; ch < 3; ++ch) acc[k][ch] = acc[k][ch] + w * Quant<float>::load(S.in[k] + t * 3 + ch);
+            ws = ws + w;
+        }
+#pragma unroll
+    for (int k = 0; k < K; ++k)
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) {
+            float v = rintf(acc[k][ch] / ws);
+            v = v > 255.0f ? 255.0f : v;
+            Quant<float>::store(S.out[k] + p * 3 + ch, v);
+        }
+}
+
 // scratch behind the packed raster buffer's clean prefix, so a bake between two renders does not cost a clear
 char *blend_scratch(wr_ctx *ctx, size_t bytes, cudaStream_t stream, int *rc)
 {
@@ -358,15 +411,10 @@ char *blend_scratch(wr_ctx *ctx, size_t bytes, cudaStream_t stream, int *rc)
     return static_cast<char *>(ctx->scratch) + wr_align256(ctx->clean_bytes);  // clean_bytes is 0 after a regrow
 }
 
-template <typename T>
-int run_inpaint(wr_ctx *ctx, const T *img, const uint8_t *mask, int mask_is_inside, int H, int W, int C, int radius,
-                T *out, cudaStream_t stream)
+// Jump flood of the known pixels of `mask` into the context scratch (opens the call's profiling stages); *seed: the
+// seed map the fill reads.
+int run_jfa(wr_ctx *ctx, const uint8_t *mask, int mask_is_inside, int H, int W, cudaStream_t stream, const int **seed)
 {
-    if (!ctx || !img || !mask || !out || H <= 0 || W <= 0 || C <= 0 || C > 4 || radius < 0 || radius > 64)
-        return WR_ERR_INVALID_ARGUMENT;
-    if (H > 16384 || W > 16384) return WR_ERR_UNSUPPORTED;
-    cudaError_t e = cudaSetDevice(ctx->device);
-    if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
     const size_t n = (size_t)H * W;
     int rc;
     char *base = blend_scratch(ctx, 2 * wr_align256(n * sizeof(int)), stream, &rc);
@@ -387,9 +435,26 @@ int run_inpaint(wr_ctx *ctx, const T *img, const uint8_t *mask, int mask_is_insi
         int *t = sa; sa = sb; sb = t;
         if (step < 1) break;
     }
+    *seed = sa;
+    return WR_OK;
+}
+
+template <typename T>
+int run_inpaint(wr_ctx *ctx, const T *img, const uint8_t *mask, int mask_is_inside, int H, int W, int C, int radius,
+                T *out, cudaStream_t stream)
+{
+    if (!ctx || !img || !mask || !out || H <= 0 || W <= 0 || C <= 0 || C > 4 || radius < 0 || radius > 64)
+        return WR_ERR_INVALID_ARGUMENT;
+    if (H > 16384 || W > 16384) return WR_ERR_UNSUPPORTED;
+    cudaError_t e = cudaSetDevice(ctx->device);
+    if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
+    const int *seed = nullptr;
+    const int rc = run_jfa(ctx, mask, mask_is_inside, H, W, stream, &seed);
+    if (rc != WR_OK) return rc;
+    const dim3 grid(wr_div_up(W, 256), H);
     wr_stage(ctx, stream, "k_inpaint_fill");
-    wr_launch(k_inpaint_fill<T>, grid, dim3(256), stream, !ctx->profiling, img, mask, mask_is_inside, (const int *)sa, H, W,
-              C, radius, out);
+    wr_launch(k_inpaint_fill<T>, grid, dim3(256), stream, !ctx->profiling, img, mask, mask_is_inside, seed, H, W, C, radius,
+              out);
     WR_CHECK_LAUNCH(ctx, "k_inpaint_fill");
     wr_stage(ctx, stream, "end");
     return WR_OK;
@@ -557,4 +622,39 @@ extern "C" int wr_uv_padding(wr_ctx *ctx, const float *attr, const uint8_t *insi
                              int radius, float *out, void *stream)
 {
     return run_inpaint<float>(ctx, attr, inside_mask, 1, H, W, C, radius, out, static_cast<cudaStream_t>(stream));
+}
+
+extern "C" int wr_uv_padding_sets(wr_ctx *ctx, const float *const *attr, const uint8_t *inside_mask, int H, int W, int K,
+                                  int radius, float *const *out, void *stream_)
+{
+    if (!ctx || !attr || !out || !inside_mask || H <= 0 || W <= 0 || K < 1 || K > WR_MAX_BAKE_SETS || radius < 0 ||
+        radius > 64)
+        return WR_ERR_INVALID_ARGUMENT;
+    PadSets S = {};
+    for (int k = 0; k < K; ++k) {
+        if (!attr[k] || !out[k]) return WR_ERR_INVALID_ARGUMENT;
+        S.in[k] = attr[k];
+        S.out[k] = out[k];
+    }
+    if (H > 16384 || W > 16384) return WR_ERR_UNSUPPORTED;
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    cudaError_t e = cudaSetDevice(ctx->device);
+    if (e != cudaSuccess) return wr_set_cuda_error(ctx, e, "cudaSetDevice");
+    const int *seed = nullptr;
+    const int rc = run_jfa(ctx, inside_mask, 1, H, W, stream, &seed);
+    if (rc != WR_OK) return rc;
+    const dim3 grid(wr_div_up(W, 256), H);
+    wr_stage(ctx, stream, "k_inpaint_fill_sets");
+    auto launch = [&](auto kernel) {
+        wr_launch(kernel, grid, dim3(256), stream, !ctx->profiling, S, inside_mask, seed, H, W, radius);
+    };
+    switch (K) {
+    case 1: launch(k_inpaint_fill_sets<1>); break;
+    case 2: launch(k_inpaint_fill_sets<2>); break;
+    case 3: launch(k_inpaint_fill_sets<3>); break;
+    default: launch(k_inpaint_fill_sets<4>); break;
+    }
+    WR_CHECK_LAUNCH(ctx, "k_inpaint_fill_sets");
+    wr_stage(ctx, stream, "end");
+    return WR_OK;
 }

@@ -299,6 +299,26 @@ def uv_padding(attr: torch.Tensor, inside_mask: torch.Tensor, radius: int, nativ
     return out
 
 
+def uv_padding_sets(attrs, inside_mask: torch.Tensor, radius: int, native_ctx=None):
+    """`uv_padding` of up to four [H,W,3] atlases against one mask in one `wr_uv_padding_sets` call: the jump flood,
+    most of a padding's cost, runs once for all of them.  Returns a list; entry k equals
+    uv_padding(attrs[k], inside_mask, radius) bit for bit."""
+    if not 1 <= len(attrs) <= _native.MAX_BAKE_SETS:
+        raise ValueError(f"uv_padding_sets: 1 to {_native.MAX_BAKE_SETS} atlases, got {len(attrs)}")
+    a = [_f32c(x.detach()) for x in attrs]
+    for x in a:
+        if x.ndim != 3 or x.shape[2] != 3 or x.shape[:2] != inside_mask.shape:
+            raise ValueError(f"uv_padding_sets: atlases [H,W,3] and inside_mask [H,W] expected, got {tuple(x.shape)}, "
+                             f"{tuple(inside_mask.shape)}")
+    m = (inside_mask != 0).contiguous().view(torch.uint8)
+    H, W = m.shape
+    out = [torch.empty_like(x) for x in a]
+    c = native_ctx if native_ctx is not None else _native.default_context(a[0].device)
+    c.check(_native.lib().wr_uv_padding_sets(c.handle, _native.ptr_array(a), _native.ptr(m), H, W, len(a), int(radius),
+                                             _native.ptr_array(out), c.stream()), "wr_uv_padding_sets")
+    return out
+
+
 def uv_blend(
     uv_precompute_output: UVPrecomputeOutput,
     uv_render_geometry_output: UVRenderGeometryOutput,
@@ -338,26 +358,45 @@ def uv_blend(
 def atlas_postprocess(blend, stitched, valid_any, pre: UVPrecomputeOutput, *, do_uv_padding=True,
                       uv_padding_radius=3, pad_unseen_area=False, poisson_blending=False, pb_solver=None,
                       pb_num_iters=1000, pb_keep_original_border=True, pb_inplace=False, pb_grad_mode="src",
-                      native_ctx=None):
+                      native_ctx=None, old_attrs=None):
     """Tail of uv_blend (uv.py:426-461) shared by the step-by-step and the fused bake: optional Poisson blend of
     the projected colours into the existing texture, then seam padding.  `blend` is the weighted view sum,
     `stitched` the same with the existing texture where no view is valid.  Where only texels outside
     `valid_any` differ (they are refilled by the padding before anything reads them) either may stand in for
-    `blend`, which is how the fused bake calls it with blend=None.  native_ctx: passed on to `uv_padding`."""
+    `blend`, which is how the fused bake calls it with blend=None.  native_ctx: passed on to `uv_padding`.
+
+    `stitched` (and `blend`) may also be lists of [H,W,3] atlases baked with the same masks (the image sets of
+    CameraProjection.project_sets).  Each padding then fills all of them in one `uv_padding_sets` call, the Poisson
+    solve runs per atlas, and a list is returned.  old_attrs: the existing texture of each set, which
+    pb_keep_original_border keeps (default pre.uv_attr for every set)."""
+    sets = not torch.is_tensor(stitched)
+
+    def pad(x, mask):
+        if sets:
+            return uv_padding_sets(x, mask, uv_padding_radius, native_ctx)
+        return uv_padding(x, mask, uv_padding_radius, native_ctx)
+
     if poisson_blending:
         assert do_uv_padding  # uv.py:427
         assert pb_solver is not None
-        padded = uv_padding(stitched if blend is None else blend, valid_any, uv_padding_radius, native_ctx)
+        padded = pad(stitched if blend is None else blend, valid_any)
         if pb_keep_original_border:
-            pb_tgt = pre.uv_attr
+            if sets:
+                pb_tgt = [pre.uv_attr] * len(stitched) if old_attrs is None else old_attrs
+            else:
+                pb_tgt = pre.uv_attr
         else:
-            pb_tgt = uv_padding(stitched, pre.uv_mask, uv_padding_radius, native_ctx)
-        out = pb_solver(padded, valid_any, pb_tgt, pb_num_iters, inplace=pb_inplace, grad_mode=pb_grad_mode)
+            pb_tgt = pad(stitched, pre.uv_mask)
+        if sets:
+            out = [pb_solver(p, valid_any, t, pb_num_iters, inplace=pb_inplace, grad_mode=pb_grad_mode)
+                   for p, t in zip(padded, pb_tgt)]
+        else:
+            out = pb_solver(padded, valid_any, pb_tgt, pb_num_iters, inplace=pb_inplace, grad_mode=pb_grad_mode)
     else:
         out = stitched
     if do_uv_padding:
         content = valid_any if pad_unseen_area else pre.uv_mask
-        out = uv_padding(out, content, uv_padding_radius, native_ctx)
+        out = pad(out, content)
     return out
 
 
@@ -377,20 +416,29 @@ class FusedBakeOutput:
 
 def fused_view_maps(ctx, mesh, cam, images, H, W, dilation):
     """View pass of the fused bake: returns (view_mask bool [Nv,H,W], geo_map, attr_map).  The shading kernel
-    writes the packed (pos, aoi_cos) map directly (no position / normal maps in HBM); wr_view_prep then only
-    adds the depth gradient and packs (rgb, depth_grad)."""
+    writes the packed (pos, aoi_cos) map directly (no position / normal maps in HBM); wr_view_prep_sets then only
+    adds the depth gradient and packs (rgb, depth_grad).
+
+    `images` is one [Nv,H,W,3] tensor (attr_map [Nv,H,W,4]) or a list of 1 to 4 of them, image sets of the same rig
+    baked together (attr_map [Nv,H,W,K,4]: set 0 is (rgb, depth_grad), set k is (rgb_k, 0)).  Float32 contiguous
+    sets are read in place."""
     dev = ctx.device
     raw = render_geometry_raw(ctx, mesh, cam, H, W, want_pos=False, want_depth=True, want_normal=False, want_geo=True,
                               depth_normalization_strategy=SimpleNormalization(**_BAKE_DEPTH))
     B = raw["geo"].shape[0]
-    images = _f32c(images)
-    if images.shape != (B, H, W, 3):
-        raise ValueError(f"images must have shape {(B, H, W, 3)}, got {tuple(images.shape)}")
-    att = torch.empty((B, H, W, 4), dtype=torch.float32, device=dev)
+    sets = [images] if torch.is_tensor(images) else list(images)
+    if not 1 <= len(sets) <= _native.MAX_BAKE_SETS:
+        raise ValueError(f"1 to {_native.MAX_BAKE_SETS} image sets, got {len(sets)}")
+    sets = [_f32c(x) for x in sets]
+    for x in sets:
+        if x.shape != (B, H, W, 3):
+            raise ValueError(f"images must have shape {(B, H, W, 3)}, got {tuple(x.shape)}")
+    shape = (B, H, W, 4) if torch.is_tensor(images) else (B, H, W, len(sets), 4)
+    att = torch.empty(shape, dtype=torch.float32, device=dev)
     c = ctx.ctx
-    status = _native.lib().wr_view_prep(c.handle, None, None, _native.ptr(raw["depth"]), None, None, _native.ptr(images),
-                                        B, H, W, int(dilation), None, None, None, _native.ptr(att), c.stream())
-    c.check(status, "wr_view_prep")
+    status = _native.lib().wr_view_prep_sets(c.handle, _native.ptr(raw["depth"]), _native.ptr_array(sets), len(sets),
+                                             B, H, W, int(dilation), None, _native.ptr(att), c.stream())
+    c.check(status, "wr_view_prep_sets")
     return raw["mask"], raw["geo"], att
 
 
@@ -417,10 +465,13 @@ def fused_unproject(ctx, pre: UVPrecomputeOutput, cam: Camera, H: int, W: int, g
                     pos_error_eps=1e-3, aoi_cos_thresh=0.1, mask_thresh=0.9, depth_grad_thresh=None,
                     first_view_dominate=False, alpha=1.0, view_weight=None, want_per_view=False,
                     accumulate_only=False, accum: Optional[torch.Tensor] = None, add_to_accum: bool = True,
-                    tex_range: Optional[tuple] = None):
+                    tex_range: Optional[tuple] = None, old_attrs=None):
     """One wr_uv_unproject launch.  Returns (attr_blend, valid_any, accum, uv_depth_grad, uv_aoi_cos).
     With accumulate_only, a given `accum` is added to (add_to_accum=True) or overwritten (False).
-    tex_range = (lo, hi): only these texels of the flattened atlas (the multi-GPU bake works chunk by chunk)."""
+    tex_range = (lo, hi): only these texels of the flattened atlas (the multi-GPU bake works chunk by chunk).
+    A K-set `att` ([Nv,H,W,K,4] from fused_view_maps with a list of image sets) bakes every set in the same launch
+    (not with accumulate_only) and attr_blend is a list of K atlases; old_attrs: the existing texture of each set,
+    a tensor or None (default pre.uv_attr for every set)."""
     dev = ctx.device
     uv_pos = _f32c(pre.uv_pos)
     uv_mask = pre.uv_mask.contiguous().view(torch.uint8)
@@ -428,6 +479,8 @@ def fused_unproject(ctx, pre: UVPrecomputeOutput, cam: Camera, H: int, W: int, g
     mvp = _f32c(cam.mvp_mtx)
     Nv = mvp.shape[0]
     a = _unproject_args(uv_pos, uv_mask, mvp, H, W, geo, att)
+    K = att.shape[3] if att.dim() == 5 else 1
+    a.attr_sets = K
     keep = [uv_pos, uv_mask, mvp]
     a.pos_error_eps, a.aoi_cos_thresh, a.mask_thresh = float(pos_error_eps), float(aoi_cos_thresh), float(mask_thresh)
     a.use_depth_grad = 0 if depth_grad_thresh is None else 1
@@ -459,16 +512,24 @@ def fused_unproject(ctx, pre: UVPrecomputeOutput, cam: Camera, H: int, W: int, g
             a.accumulate = 1 if add_to_accum else 0
         a.accum = _native.ptr(accum)
     else:
-        old = pre.uv_attr
-        if old is not None:
-            old = _f32c(old)
-            if old.shape != (Hu, Wu, 3):
-                raise ValueError(f"existing texture must be {(Hu, Wu, 3)}, got {tuple(old.shape)}")
-            keep.append(old)
-            a.old_attr = _native.ptr(old)
-        out_attr = torch.empty((Hu, Wu, 3), dtype=torch.float32, device=dev)
+        olds = [pre.uv_attr] * K if old_attrs is None else list(old_attrs)
+        if len(olds) != K:
+            raise ValueError(f"old_attrs must have one entry per image set ({K}), got {len(olds)}")
+        outs = []
+        for k, old in enumerate(olds):
+            if old is not None:
+                old = _f32c(old)
+                if old.shape != (Hu, Wu, 3):
+                    raise ValueError(f"existing texture must be {(Hu, Wu, 3)}, got {tuple(old.shape)}")
+                keep.append(old)
+            outs.append(torch.empty((Hu, Wu, 3), dtype=torch.float32, device=dev))
+            if k == 0:
+                a.old_attr, a.out_attr = _native.ptr(old), _native.ptr(outs[0])
+            else:
+                a.old_attr_more[k - 1], a.out_attr_more[k - 1] = _native.ptr(old), _native.ptr(outs[k])
+        out_attr = outs if att.dim() == 5 else outs[0]
         out_any = torch.empty((Hu, Wu), dtype=torch.uint8, device=dev)
-        a.out_attr, a.out_valid_any = _native.ptr(out_attr), _native.ptr(out_any)
+        a.out_valid_any = _native.ptr(out_any)
     if tex_range is not None:
         a.tex_lo, a.tex_hi = int(tex_range[0]), int(tex_range[1])
     c = ctx.ctx
