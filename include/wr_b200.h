@@ -66,7 +66,7 @@ const char *wr_status_string(int status);
 const char *wr_ctx_last_error(const wr_ctx *ctx);
 /* Version of this header's ABI (struct layouts included).  wr_version() returns the value the LIBRARY was built with:
  * a caller compiled against another header must not go on (its argument structs have a different layout). */
-#define WR_B200_ABI_VERSION 104
+#define WR_B200_ABI_VERSION 105
 int wr_version(void);
 
 /* One context per (device, stream in flight).  Not thread-safe, like the reference's contexts. */
@@ -120,6 +120,9 @@ int wr_tangent_space_normals(wr_ctx *ctx, const float *normal, const float *tang
 /* depth normalisers of render.py:164-217 */
 enum { WR_DEPTH_NONE = 0, WR_DEPTH_CONTROLNET = 1, WR_DEPTH_ZERO123PP = 2, WR_DEPTH_SIMPLE = 3 };
 
+/* element type of wr_render's position, depth, normal, tangent and attribute maps */
+enum { WR_DTYPE_F32 = 0, WR_DTYPE_F16 = 1, WR_DTYPE_BF16 = 2 };
+
 typedef struct wr_render_args {
     /* mesh */
     const float *v_pos;       /* [V,3] */
@@ -147,7 +150,8 @@ typedef struct wr_render_args {
     float normal_bg[3];
     float tangent_bg[3];
     float attr_bg;
-    /* outputs, each may be NULL */
+    /* outputs, each may be NULL; out_pos / out_depth / out_normal / out_tangent / out_attr hold elements of out_dtype
+       (declared float: cast a half buffer's pointer) */
     uint8_t *out_mask;        /* [B,H,W] 0/1 */
     float *out_pos;           /* [B,H,W,3] */
     float *out_depth;         /* [B,H,W] */
@@ -161,6 +165,10 @@ typedef struct wr_render_args {
        caller that renders groups of views on several streams (graph.RenderGraph(view_lanes, stagger)) makes group
        k + 1 wait for it, so that its issue-bound raster passes run next to the store-bound shading pass of group k. */
     void *raster_done_event;
+    /* Element type of out_pos / out_depth / out_normal / out_tangent / out_attr; out_geo, out_rast and out_tri_id are
+       unaffected.  Values are computed in float32 as for WR_DTYPE_F32 and rounded to nearest even on the store, so a
+       16-bit map equals the float32 map converted (NaN payloads aside).  Any other value: WR_ERR_INVALID_ARGUMENT. */
+    int out_dtype;            /* WR_DTYPE_F32 = 0 (default), WR_DTYPE_F16, WR_DTYPE_BF16 */
 } wr_render_args;
 
 int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream);

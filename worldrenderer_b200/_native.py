@@ -31,6 +31,7 @@ SYMBOLS = [
 ]
 
 DEPTH_NONE, DEPTH_CONTROLNET, DEPTH_ZERO123PP, DEPTH_SIMPLE = 0, 1, 2, 3
+DTYPE_F32, DTYPE_F16, DTYPE_BF16 = 0, 1, 2   # wr_render_args.out_dtype
 
 
 class RenderArgs(ctypes.Structure):
@@ -50,6 +51,7 @@ class RenderArgs(ctypes.Structure):
         ("out_normal", ctypes.c_void_p), ("out_tangent", ctypes.c_void_p), ("out_geo", ctypes.c_void_p), ("out_attr", ctypes.c_void_p), ("out_tri_id", ctypes.c_void_p),
         ("out_rast", ctypes.c_void_p),
         ("raster_done_event", ctypes.c_void_p),
+        ("out_dtype", ctypes.c_int),
     ]
 
 
@@ -76,7 +78,7 @@ class UnprojectArgs(ctypes.Structure):
     ]
 
 
-ABI_VERSION = 104   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
+ABI_VERSION = 105   # include/wr_b200.h WR_B200_ABI_VERSION (the ctypes structures below mirror that header)
 MAX_P2P_RANKS = 16
 
 

@@ -19,8 +19,16 @@
 //   k_depth_finalize  second depth pass for normalisers that need the per-view min / max (covered pixels only:
 //                     the constant background value is written by k_shade).
 //
+// Output element type (wr_render_args.out_dtype): float, __half or __nv_bfloat16 behind the position, depth, normal,
+// tangent and attribute maps.  Every value is computed in float32 exactly as for float output and rounded to nearest
+// even on the store only, so a half map equals the float map cast by torch.  A two-pass depth normaliser in half
+// precision keeps the raw float32 view depth in scratch for k_depth_finalize, which writes the half map.
+//
 // The shading kernel resets every packed entry it consumes to WR_EMPTY_PIXEL, which leaves the
 // buffer clean for the next call (no clear pass).
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 #include "texture.cuh"
 
@@ -37,7 +45,24 @@ struct ShadeParams {
     int wide_ok;                 // W % 4 == 0 and 16-byte aligned pos / normal maps: background rows may use 16-byte stores
     int bg_final;                // two-pass depth whose background value is a constant (controlnet, zero123++):
                                  // written here, k_depth_finalize then only touches covered pixels
+    float *depth_raw;            // [B,H,W] two-pass view depth read by k_depth_finalize: out_depth for float output,
+                                 // scratch otherwise
 };
+
+// store conversion of the output maps: round to nearest even, as torch's casts
+template <typename T> __device__ __forceinline__ T to_out(float x);
+template <> __device__ __forceinline__ float to_out<float>(float x) { return x; }
+template <> __device__ __forceinline__ __half to_out<__half>(float x) { return __float2half_rn(x); }
+template <> __device__ __forceinline__ __nv_bfloat16 to_out<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
+
+// two 16-bit elements in one 32-bit word, `lo` at the lower address
+template <typename T> __device__ __forceinline__ uint32_t pack2(T lo, T hi)
+{
+    uint16_t a, b;
+    memcpy(&a, &lo, 2);
+    memcpy(&b, &hi, 2);
+    return (uint32_t)a | ((uint32_t)b << 16);
+}
 
 struct PixelGeo {
     float px, py, pz;   // world position (zeros on background)
@@ -221,11 +246,18 @@ constexpr int kOutsSimpleDepth = kOutNormal | kOutDepth;                  // mas
 constexpr int kOutsBakeView = kOutGeo | kOutDepth;                        // mask + (pos, aoi_cos) + simple depth
 
 // One column strip of kShadeRows pixels per thread.  grid = (ceil(W/128), ceil(H/kShadeRows), B), 128 threads.
-template <int OUTS, bool PACKED>
+// T: element type of the position, depth, normal, tangent and attribute maps.
+template <int OUTS, bool PACKED, typename T>
 __global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeParams P)
 {
     const wr_render_args &A = P.a;
     constexpr bool kGeneric = OUTS < 0;
+    constexpr bool kF32 = sizeof(T) == 4;
+    T *const out_pos = reinterpret_cast<T *>(A.out_pos);
+    T *const out_depth = reinterpret_cast<T *>(A.out_depth);
+    T *const out_normal = reinterpret_cast<T *>(A.out_normal);
+    T *const out_tangent = reinterpret_cast<T *>(A.out_tangent);
+    T *const out_attr = reinterpret_cast<T *>(A.out_attr);
     const bool has_mask = kGeneric ? (P.mask != nullptr) : true;
     const bool has_geo = kGeneric ? (A.out_geo != nullptr) : ((OUTS & kOutGeo) != 0);
     const bool has_pos = kGeneric ? (A.out_pos != nullptr) : !has_geo;
@@ -294,15 +326,40 @@ __global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeP
                 const float t2 = e == 0 ? nbz : (e == 1 ? nbx : nby);
                 n4 = make_float4(t0, t1, t2, t0);
             }
-            for (int k = 0; k < nrows; ++k) {
-                const size_t o = o0 + (size_t)k * W;
-                const size_t row4 = (3 * (o - lane)) >> 2;  // float4 index of the warp's row segment
-                if (lane < 24) {
-                    reinterpret_cast<float4 *>(A.out_pos)[row4 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (has_normal) reinterpret_cast<float4 *>(A.out_normal)[row4 + lane] = n4;
+            if constexpr (kF32) {
+                for (int k = 0; k < nrows; ++k) {
+                    const size_t o = o0 + (size_t)k * W;
+                    const size_t row4 = (3 * (o - lane)) >> 2;  // float4 index of the warp's row segment
+                    if (lane < 24) {
+                        reinterpret_cast<float4 *>(A.out_pos)[row4 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
+                        if (has_normal) reinterpret_cast<float4 *>(A.out_normal)[row4 + lane] = n4;
+                    }
+                    P.mask[o] = 0;
+                    if (has_depth) A.out_depth[o] = two_pass ? (bg_final ? A.depth_bg : d_bg) : A.depth_bg;
                 }
-                P.mask[o] = 0;
-                if (has_depth) A.out_depth[o] = two_pass ? (bg_final ? A.depth_bg : d_bg) : A.depth_bg;
+            } else {
+                // 16-bit maps: a row segment of 96 elements is 12 x 16 bytes, elements 8*lane .. 8*lane+7 per lane
+                // (W % 8 == 0, see wide_ok); n4 holds the triple rotated for element 4*lane, this one for 8*lane
+                const int e = (8 * (int)lane) % 3;
+                const T h0 = to_out<T>(e == 0 ? nbx : (e == 1 ? nby : nbz));
+                const T h1 = to_out<T>(e == 0 ? nby : (e == 1 ? nbz : nbx));
+                const T h2 = to_out<T>(e == 0 ? nbz : (e == 1 ? nbx : nby));
+                const uint4 n8 = make_uint4(pack2(h0, h1), pack2(h2, h0), pack2(h1, h2), pack2(h0, h1));
+                const T dbg = to_out<T>(A.depth_bg);
+#pragma unroll 1  // unrolled, it pushes the specialised 16-bit instantiations past 64 registers (spills)
+                for (int k = 0; k < nrows; ++k) {
+                    const size_t o = o0 + (size_t)k * W;
+                    const size_t row8 = (3 * (o - lane)) >> 3;  // 16-byte index of the warp's row segment
+                    if (lane < 12) {
+                        reinterpret_cast<uint4 *>(out_pos)[row8 + lane] = make_uint4(0u, 0u, 0u, 0u);
+                        if (has_normal) reinterpret_cast<uint4 *>(out_normal)[row8 + lane] = n8;
+                    }
+                    P.mask[o] = 0;
+                    if (has_depth) {
+                        if (two_pass && !bg_final) P.depth_raw[o] = d_bg;
+                        else out_depth[o] = dbg;
+                    }
+                }
             }
             if (two_pass) lo = d_bg;
             goto publish;
@@ -350,15 +407,15 @@ __global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeP
             aoi = fminf(fmaxf(aoi, 0.0f), 1.0f);
             reinterpret_cast<float4 *>(A.out_geo)[o] = make_float4(g.px, g.py, g.pz, aoi);
         }
-        if (has_pos) { float *d = A.out_pos + 3 * o; d[0] = g.px; d[1] = g.py; d[2] = g.pz; }
-        if (has_normal) { float *d = A.out_normal + 3 * o; d[0] = g.nx; d[1] = g.ny; d[2] = g.nz; }
-        if (has_tangent) { float *d = A.out_tangent + 3 * o; d[0] = g.tx; d[1] = g.ty; d[2] = g.tz; }
+        if (has_pos) { T *d = out_pos + 3 * o; d[0] = to_out<T>(g.px); d[1] = to_out<T>(g.py); d[2] = to_out<T>(g.pz); }
+        if (has_normal) { T *d = out_normal + 3 * o; d[0] = to_out<T>(g.nx); d[1] = to_out<T>(g.ny); d[2] = to_out<T>(g.nz); }
+        if (has_tangent) { T *d = out_tangent + 3 * o; d[0] = to_out<T>(g.tx); d[1] = to_out<T>(g.ty); d[2] = to_out<T>(g.tz); }
         if (has_id) A.out_tri_id[o] = id;
         if (has_rast)
             reinterpret_cast<float4 *>(A.out_rast)[o] =
                 covered ? make_float4(g.u, g.v, g.zw, (float)(id + 1)) : make_float4(0.f, 0.f, 0.f, 0.f);
         if (has_attr) {
-            float *d = A.out_attr + (size_t)A.TC * o;
+            T *d = out_attr + (size_t)A.TC * o;
             if (covered) {
                 const int t0 = __ldg(A.tri_tex + 3 * (size_t)id), t1 = __ldg(A.tri_tex + 3 * (size_t)id + 1),
                           t2 = __ldg(A.tri_tex + 3 * (size_t)id + 2);
@@ -371,10 +428,11 @@ __global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeP
                 for (int c0 = 0; c0 < A.TC; c0 += 4) {
                     float acc[4];
                     sample_texture<4>(A.texture + c0, A.TH, A.TW, A.TC, min(4, A.TC - c0), tu, tv, A.tex_filter, 0, acc);
-                    for (int j = 0; j < 4 && c0 + j < A.TC; ++j) d[c0 + j] = acc[j];
+                    for (int j = 0; j < 4 && c0 + j < A.TC; ++j) d[c0 + j] = to_out<T>(acc[j]);
                 }
             } else {
-                for (int j = 0; j < A.TC; ++j) d[j] = A.attr_bg;
+                const T bg = to_out<T>(A.attr_bg);
+                for (int j = 0; j < A.TC; ++j) d[j] = bg;
             }
         }
         if (has_depth) {
@@ -382,9 +440,11 @@ __global__ void __launch_bounds__(kShadeThreads, kShadeMinBlocks) k_shade(ShadeP
             const float zv = ((wz0 * g.px + wz1 * g.py) + wz2 * g.pz) + wz3;
             const float d = -zv;
             if (!two_pass) {
-                A.out_depth[o] = covered ? apply_simple(d, A.depth_p0, A.depth_p1, A.depth_clamp) : A.depth_bg;
+                out_depth[o] = to_out<T>(covered ? apply_simple(d, A.depth_p0, A.depth_p1, A.depth_clamp) : A.depth_bg);
             } else {
-                A.out_depth[o] = (bg_final && !covered) ? A.depth_bg : d;
+                if constexpr (kF32) A.out_depth[o] = (bg_final && !covered) ? A.depth_bg : d;
+                else if (bg_final && !covered) out_depth[o] = to_out<T>(A.depth_bg);  // k_depth_finalize skips it
+                else P.depth_raw[o] = d;
                 lo = fminf(lo, d);
                 if (covered) hi = fmaxf(hi, d);
             }
@@ -424,20 +484,25 @@ __device__ __forceinline__ float finalize_one(float d, bool covered, float lo, f
     return x;
 }
 
-__global__ void __launch_bounds__(256) k_depth_finalize(float *depth, const uint8_t *mask, const uint32_t *range,
-                                                        long long npix_view, int mode, float p0, float p1, float bg,
-                                                        int vec, int bg_final)
+// Reads the float32 view depth `raw` and writes `depth` (the same buffer for float output).
+template <typename T>
+__global__ void __launch_bounds__(256) k_depth_finalize(const float *raw, T *depth, const uint8_t *mask,
+                                                        const uint32_t *range, long long npix_view, int mode, float p0,
+                                                        float p1, float bg, int vec, int bg_final)
 {
     wr_pdl_wait();
     const int b = blockIdx.y;
-    float *dv = depth + (size_t)b * npix_view;
+    T *dv = depth + (size_t)b * npix_view;
+    const float *rv;
+    if constexpr (sizeof(T) == 4) rv = dv;  // in place, as one pointer: the float kernel keeps its code
+    else rv = raw + (size_t)b * npix_view;
     const uint8_t *mv = mask + (size_t)b * npix_view;
     const long long gi = (long long)blockIdx.x * 256 + threadIdx.x;  // group of 4 pixels
     if (vec) {
         if (gi >= (npix_view >> 2)) return;
         const uchar4 m = reinterpret_cast<const uchar4 *>(mv)[gi];
         if (bg_final && !(m.x | m.y | m.z | m.w)) return;
-        const float4 d = reinterpret_cast<const float4 *>(dv)[gi];
+        const float4 d = reinterpret_cast<const float4 *>(rv)[gi];
         const float lo = wr_ordered_float(~range[4 * b]);
         const uint32_t hik = range[4 * b + 1];
         const float hi = hik == 0u ? lo : wr_ordered_float(hik);  // no covered pixel: filled image is constant lo
@@ -447,7 +512,11 @@ __global__ void __launch_bounds__(256) k_depth_finalize(float *depth, const uint
         o.y = finalize_one(d.y, m.y, lo, den, mode, p0, p1, bg);
         o.z = finalize_one(d.z, m.z, lo, den, mode, p0, p1, bg);
         o.w = finalize_one(d.w, m.w, lo, den, mode, p0, p1, bg);
-        reinterpret_cast<float4 *>(dv)[gi] = o;
+        if constexpr (sizeof(T) == 4)
+            reinterpret_cast<float4 *>(dv)[gi] = o;
+        else  // one 8-byte store
+            reinterpret_cast<uint2 *>(dv)[gi] = make_uint2(pack2(to_out<T>(o.x), to_out<T>(o.y)),
+                                                           pack2(to_out<T>(o.z), to_out<T>(o.w)));
     } else {
         const float lo = wr_ordered_float(~range[4 * b]);
         const uint32_t hik = range[4 * b + 1];
@@ -455,9 +524,40 @@ __global__ void __launch_bounds__(256) k_depth_finalize(float *depth, const uint
         const float den = (hi - lo) + 1e-5f;
         for (int j = 0; j < 4; ++j) {
             const long long i = gi * 4 + j;
-            if (i < npix_view) dv[i] = finalize_one(dv[i], mv[i] != 0, lo, den, mode, p0, p1, bg);
+            if (i < npix_view) dv[i] = to_out<T>(finalize_one(rv[i], mv[i] != 0, lo, den, mode, p0, p1, bg));
         }
     }
+}
+
+// One instantiation per output set (see kOuts*), vertex source and output element type.
+template <typename T>
+void launch_shade(const ShadeParams &P, bool use_pack, bool plain, bool two_pass, bool bake, dim3 grid, dim3 block,
+                  cudaStream_t stream, bool pdl)
+{
+    if (use_pack) {
+        if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, true, T>, grid, block, stream, pdl, P);
+        else if (plain) wr_launch(k_shade<kOutsSimpleDepth, true, T>, grid, block, stream, pdl, P);
+        else if (bake) wr_launch(k_shade<kOutsBakeView, true, T>, grid, block, stream, pdl, P);
+        else wr_launch(k_shade<-1, true, T>, grid, block, stream, pdl, P);
+    } else {
+        if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, false, T>, grid, block, stream, pdl, P);
+        else if (plain) wr_launch(k_shade<kOutsSimpleDepth, false, T>, grid, block, stream, pdl, P);
+        else if (bake) wr_launch(k_shade<kOutsBakeView, false, T>, grid, block, stream, pdl, P);
+        else wr_launch(k_shade<-1, false, T>, grid, block, stream, pdl, P);
+    }
+}
+
+template <typename T>
+void launch_finalize(const wr_render_args &A, const ShadeParams &P, cudaStream_t stream, bool pdl)
+{
+    const long long npv = (long long)A.H * A.W;
+    T *const depth = reinterpret_cast<T *>(A.out_depth);
+    const int vec = (npv & 3) == 0 && (reinterpret_cast<uintptr_t>(P.depth_raw) & 15u) == 0 &&
+                    (reinterpret_cast<uintptr_t>(depth) & (4 * sizeof(T) - 1)) == 0 &&
+                    (reinterpret_cast<uintptr_t>(P.mask) & 3u) == 0;
+    wr_launch(k_depth_finalize<T>, dim3(wr_div_up(wr_div_up(npv, 4), 256), A.B), dim3(256), stream, pdl,
+              (const float *)P.depth_raw, depth, (const uint8_t *)P.mask, (const uint32_t *)P.range, npv, A.depth_mode,
+              A.depth_p0, A.depth_p1, A.depth_bg, vec, P.bg_final);
 }
 
 }  // namespace
@@ -467,6 +567,7 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
     if (!ctx || !args) return WR_ERR_INVALID_ARGUMENT;
     const wr_render_args &A = *args;
     if (A.B < 0 || A.V < 0 || A.F < 0 || A.H <= 0 || A.W <= 0 || A.H > 8192 || A.W > 8192) return WR_ERR_INVALID_ARGUMENT;
+    if (A.out_dtype < WR_DTYPE_F32 || A.out_dtype > WR_DTYPE_BF16) return WR_ERR_INVALID_ARGUMENT;
     if (A.F >= (1 << 30)) return WR_ERR_UNSUPPORTED;
     if (A.out_rast && A.F > (1 << 24)) return WR_ERR_UNSUPPORTED;  // (float)(id + 1) is exact up to 2^24 faces
     if (A.B == 0) return WR_OK;
@@ -491,18 +592,21 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
     void *extra = nullptr;
     wr_stage_begin(ctx);
     const size_t mask_bytes = (two_pass && !A.out_mask) ? wr_align256(npix) : 0;
+    const size_t esize = A.out_dtype == WR_DTYPE_F32 ? 4 : 2;
+    // float32 view depth of a two-pass normaliser with 16-bit output, behind the mask in the extra scratch
+    const size_t raw_bytes = (two_pass && esize != 4) ? wr_align256(npix * 4) : 0;
     const bool want_nrm = A.v_nrm && (A.out_normal || A.out_geo);
     VertexPack pack;
     pack.v_nrm = want_nrm ? A.v_nrm : nullptr;
     pack.Vn = A.Vn;
-    pack.offset = mask_bytes;
+    pack.offset = mask_bytes + raw_bytes;
     // 16-byte vertex records pay off when many pixels gather from few vertices (config A: 45.4 vs 47.4 us in
     // k_shade); for a mesh of sub-pixel triangles writing them costs more than they save (config B: +3.3 us)
     const bool use_pack = (long long)A.B * A.H * A.W >= 32ll * ((long long)A.V + (want_nrm ? A.Vn : 0));
     pack.pos4 = nullptr;
     pack.nrm4 = nullptr;
     int rc = wr_run_raster(ctx, src, A.B, A.tri, A.F, nullptr, A.H, A.W,
-                           mask_bytes + (use_pack ? wr_vertex_pack_bytes(A.V, A.Vn, want_nrm) : 0), &res, &extra,
+                           mask_bytes + raw_bytes + (use_pack ? wr_vertex_pack_bytes(A.V, A.Vn, want_nrm) : 0), &res, &extra,
                            stream, use_pack ? &pack : nullptr);
     if (rc != WR_OK) return rc;
     if (A.raster_done_event) {
@@ -517,9 +621,12 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
     P.range = reinterpret_cast<uint32_t *>(res.view_stats);
     P.pos4 = pack.pos4;
     P.nrm4 = pack.nrm4;
-    P.wide_ok = (A.W & 3) == 0 && (reinterpret_cast<uintptr_t>(A.out_pos) & 15u) == 0 &&
+    // a warp's background row segment (32 pixels x 3 elements) starts on a 16-byte boundary: W % 4 == 0 for float,
+    // W % 8 == 0 for 16-bit maps
+    P.wide_ok = (A.W % (int)(16 / esize)) == 0 && (reinterpret_cast<uintptr_t>(A.out_pos) & 15u) == 0 &&
                 (reinterpret_cast<uintptr_t>(A.out_normal) & 15u) == 0;
     P.bg_final = two_pass && (A.depth_mode == WR_DEPTH_CONTROLNET || A.depth_mode == WR_DEPTH_ZERO123PP);
+    P.depth_raw = raw_bytes ? reinterpret_cast<float *>(static_cast<char *>(extra) + mask_bytes) : A.out_depth;
     wr_stage(ctx, stream, "k_shade");
     {
         const dim3 grid(wr_div_up(A.W, kShadeThreads), wr_div_up(A.H, kShadeRows), A.B);
@@ -529,28 +636,17 @@ extern "C" int wr_render(wr_ctx *ctx, const wr_render_args *args, void *stream_)
         // dependent launch only when the raster stages were launched (the chain's first kernel is a plain launch)
         const bool pdl = !ctx->profiling && A.F > 0 && A.V > 0;
         const dim3 block(kShadeThreads);
-        if (use_pack) {
-            if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, true>, grid, block, stream, pdl, P);
-            else if (plain) wr_launch(k_shade<kOutsSimpleDepth, true>, grid, block, stream, pdl, P);
-            else if (bake) wr_launch(k_shade<kOutsBakeView, true>, grid, block, stream, pdl, P);
-            else wr_launch(k_shade<-1, true>, grid, block, stream, pdl, P);
-        } else {
-            if (plain && two_pass) wr_launch(k_shade<kOutsRenderDefault, false>, grid, block, stream, pdl, P);
-            else if (plain) wr_launch(k_shade<kOutsSimpleDepth, false>, grid, block, stream, pdl, P);
-            else if (bake) wr_launch(k_shade<kOutsBakeView, false>, grid, block, stream, pdl, P);
-            else wr_launch(k_shade<-1, false>, grid, block, stream, pdl, P);
-        }
+        if (A.out_dtype == WR_DTYPE_F16) launch_shade<__half>(P, use_pack, plain, two_pass, bake, grid, block, stream, pdl);
+        else if (A.out_dtype == WR_DTYPE_BF16) launch_shade<__nv_bfloat16>(P, use_pack, plain, two_pass, bake, grid, block, stream, pdl);
+        else launch_shade<float>(P, use_pack, plain, two_pass, bake, grid, block, stream, pdl);
     }
     WR_CHECK_LAUNCH(ctx, "k_shade");
     wr_raster_consumed(ctx, &res);
     if (two_pass) {
-        const long long npv = (long long)A.H * A.W;
-        const int vec = (npv & 3) == 0 && (reinterpret_cast<uintptr_t>(A.out_depth) & 15u) == 0 &&
-                        (reinterpret_cast<uintptr_t>(P.mask) & 3u) == 0;
         wr_stage(ctx, stream, "k_depth_finalize");
-        wr_launch(k_depth_finalize, dim3(wr_div_up(wr_div_up(npv, 4), 256), A.B), dim3(256), stream, !ctx->profiling,
-                  A.out_depth, (const uint8_t *)P.mask, (const uint32_t *)P.range, npv, A.depth_mode, A.depth_p0,
-                  A.depth_p1, A.depth_bg, vec, P.bg_final);
+        if (A.out_dtype == WR_DTYPE_F16) launch_finalize<__half>(A, P, stream, !ctx->profiling);
+        else if (A.out_dtype == WR_DTYPE_BF16) launch_finalize<__nv_bfloat16>(A, P, stream, !ctx->profiling);
+        else launch_finalize<float>(A, P, stream, !ctx->profiling);
         WR_CHECK_LAUNCH(ctx, "k_depth_finalize");
     }
     wr_stage(ctx, stream, "end");

@@ -27,6 +27,9 @@ from .mesh import TexturedMesh
 
 _FILTER_MODES = {"nearest": 0, "linear": 1, "auto": 1}
 _BOUNDARY_MODES = {"wrap": 0, "clamp": 1, "zero": 2}
+# render(output_dtype=...): element type of the pos / depth / normal / tangent / attr maps (wr_render_args.out_dtype)
+_OUTPUT_DTYPES = {torch.float32: _native.DTYPE_F32, torch.float16: _native.DTYPE_F16,
+                  torch.bfloat16: _native.DTYPE_BF16}
 
 
 @dataclass
@@ -271,11 +274,15 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
                         want_rast=False, want_tangent=False, tangent_background=0.0, want_geo=False,
                         depth_normalization_strategy=None, normal_background=0.0,
                         attr_background=0.5, texture_override=None, texture_filter_mode="linear", out_buffers=None,
-                        raster_done_event=None):
+                        raster_done_event=None, output_dtype=torch.float32):
     """One wr_render call.  Returns a dict of tensors; `mask` is uint8 0/1 (callers view it as bool).
     out_buffers: optional {name: preallocated contiguous tensor} written instead of fresh allocations (RenderGraph
     renders groups of views into slices of one output).  raster_done_event: a recorded-at-least-once torch.cuda.Event,
-    re-recorded by the library between the raster passes and the shading pass (wr_render_args.raster_done_event)."""
+    re-recorded by the library between the raster passes and the shading pass (wr_render_args.raster_done_event).
+    output_dtype: float32, float16 or bfloat16 for pos / depth / normal / tangent / attr (geo stays float32); the
+    result equals the float32 maps cast to it."""
+    if output_dtype not in _OUTPUT_DTYPES:
+        raise ValueError(f"output_dtype must be torch.float32, torch.float16 or torch.bfloat16, got {output_dtype!r}")
     dev = ctx.device
 
     def _new(name, shape, dtype):
@@ -295,7 +302,22 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
     w2c = _f32c(cam.w2c)
     ctx._check_device(v_pos, tri, mvp, w2c)
     B, H, W = mvp.shape[0], int(height), int(width)
+    post = _depth_kernel_params(depth_normalization_strategy)[5] if want_depth else None
+    nbg = _background_triplet(normal_background, "normal_background") if (want_normal or want_geo) else None
+    tbg = _background_triplet(tangent_background, "tangent_background") if want_tangent else None
+    abg_is_tensor = want_attr and isinstance(attr_background, torch.Tensor) and attr_background.numel() != 1
+    # A map that torch post-processes (user-defined depth strategy, per-pixel background tensor) is computed in float32
+    # and cast once at the end, so that the result still equals the float32 render cast to output_dtype.
+    torch_tail = post is not None or (want_normal and nbg is None) or (want_tangent and tbg is None) or abg_is_tensor
+    map_dtype = torch.float32 if torch_tail else output_dtype
+
+    def _map(name, shape):
+        if map_dtype != output_dtype:   # not the caller's buffer: the cast at the end allocates the result
+            return torch.empty(shape, dtype=map_dtype, device=dev)
+        return _new(name, shape, map_dtype)
+
     a = _native.RenderArgs()
+    a.out_dtype = _OUTPUT_DTYPES[map_dtype]
     keep = [v_pos, tri, mvp, w2c]
     a.v_pos, a.tri, a.V, a.F = _native.ptr(v_pos), _native.ptr(tri), v_pos.shape[0], tri.shape[0]
     a.mvp, a.w2c, a.B, a.H, a.W = _native.ptr(mvp), _native.ptr(w2c), B, H, W
@@ -303,13 +325,12 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
     out["mask"] = _new("mask", (B, H, W), torch.uint8)
     a.out_mask = _native.ptr(out["mask"])
     if want_pos:
-        out["pos"] = _new("pos", (B, H, W, 3), torch.float32)
+        out["pos"] = _map("pos", (B, H, W, 3))
         a.out_pos = _native.ptr(out["pos"])
-    post = None
     if want_depth:
-        mode, p0, p1, clamp, bg, post = _depth_kernel_params(depth_normalization_strategy)
+        mode, p0, p1, clamp, bg, _ = _depth_kernel_params(depth_normalization_strategy)
         a.depth_mode, a.depth_p0, a.depth_p1, a.depth_clamp, a.depth_bg = mode, p0, p1, clamp, bg
-        out["depth"] = _new("depth", (B, H, W), torch.float32)
+        out["depth"] = _map("depth", (B, H, W))
         a.out_depth = _native.ptr(out["depth"])
     if want_geo or want_normal or want_tangent:
         # the kernel reads tri_nrm[3 * id] for every covered pixel: one row per face of t_pos_idx, or an
@@ -324,8 +345,7 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
         same_faces = mesh._stitched_t_pos_idx is None or mesh._stitched_t_pos_idx is mesh.t_pos_idx
         a.v_nrm, a.Vn = _native.ptr(v_nrm), v_nrm.shape[0]
         a.tri_nrm = None if same_faces else _native.ptr(tri_n)
-        nbg = _background_triplet(normal_background, "normal_background") or [0.0, 0.0, 0.0]
-        a.normal_bg = (ctypes.c_float * 3)(*nbg)
+        a.normal_bg = (ctypes.c_float * 3)(*(nbg or [0.0, 0.0, 0.0]))
         out["geo"] = _new("geo", (B, H, W, 4), torch.float32)
         a.out_geo = _native.ptr(out["geo"])
     nbg_tensor = None
@@ -338,11 +358,10 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
         same_faces = mesh._stitched_t_pos_idx is None or mesh._stitched_t_pos_idx is mesh.t_pos_idx
         a.v_nrm, a.Vn = _native.ptr(v_nrm), v_nrm.shape[0]
         a.tri_nrm = None if same_faces else _native.ptr(tri_n)
-        nbg = _background_triplet(normal_background, "normal_background")
         if nbg is None:
             nbg_tensor, nbg = normal_background, [0.0, 0.0, 0.0]
         a.normal_bg = (ctypes.c_float * 3)(*nbg)
-        out["normal"] = _new("normal", (B, H, W, 3), torch.float32)
+        out["normal"] = _map("normal", (B, H, W, 3))
         a.out_normal = _native.ptr(out["normal"])
     tbg_tensor = None
     if want_tangent:
@@ -356,11 +375,10 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
         same_faces = mesh._stitched_t_pos_idx is None or mesh._stitched_t_pos_idx is mesh.t_pos_idx
         a.v_tang, a.Vn = _native.ptr(v_tang), v_tang.shape[0]
         a.tri_nrm = None if same_faces else _native.ptr(tri_n)
-        tbg = _background_triplet(tangent_background, "tangent_background")
         if tbg is None:
             tbg_tensor, tbg = tangent_background, [0.0, 0.0, 0.0]
         a.tangent_bg = (ctypes.c_float * 3)(*tbg)
-        out["tangent"] = _new("tangent", (B, H, W, 3), torch.float32)
+        out["tangent"] = _map("tangent", (B, H, W, 3))
         a.out_tangent = _native.ptr(out["tangent"])
     abg_tensor = None
     if want_attr:
@@ -377,11 +395,11 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
         a.v_tex, a.tri_tex, a.Vt = _native.ptr(v_tex), _native.ptr(tri_t), v_tex.shape[0]
         a.texture, a.TH, a.TW, a.TC = _native.ptr(tex), tex.shape[0], tex.shape[1], tex.shape[2]
         a.tex_filter = _FILTER_MODES[texture_filter_mode]
-        if isinstance(attr_background, torch.Tensor) and attr_background.numel() != 1:
+        if abg_is_tensor:
             abg_tensor, a.attr_bg = attr_background, 0.0
         else:
             a.attr_bg = float(attr_background)
-        out["attr"] = _new("attr", (B, H, W, tex.shape[2]), torch.float32)
+        out["attr"] = _map("attr", (B, H, W, tex.shape[2]))
         a.out_attr = _native.ptr(out["attr"])
     if want_tri_id:
         out["tri_id"] = _new("tri_id", (B, H, W), torch.int32)
@@ -407,6 +425,10 @@ def render_geometry_raw(ctx: NVDiffRastContextWrapper, mesh: TexturedMesh, cam: 
     if abg_tensor is not None:
         bgv = torch.ones_like(out["attr"]) * abg_tensor.to(out["attr"])
         out["attr"] = torch.where(mask_bool[..., None], out["attr"], bgv)
+    if map_dtype != output_dtype:
+        for name in ("pos", "depth", "normal", "tangent", "attr"):
+            if name in out:
+                out[name] = out[name].to(output_dtype)
     out["mask"] = mask_bool
     return out
 
@@ -428,10 +450,16 @@ def render(
     tangent_background: Union[float, torch.Tensor] = 0.0,
     texture_override=None,
     texture_filter_mode: str = "linear",
+    output_dtype: torch.dtype = torch.float32,
     _out_buffers=None,
     _raster_done_event=None,
 ) -> RenderOutput:
-    """Same signature and outputs as the reference render() (render.py:220-286)."""
+    """Same signature and outputs as the reference render() (render.py:220-286), plus `output_dtype`.
+
+    output_dtype: torch.float32 (default), torch.float16 or torch.bfloat16 -- element type of pos, depth, normal,
+    tangent and attr (mask stays bool).  Everything is computed in float32 and rounded to nearest even when stored,
+    so the maps equal `render(...)` with each float map cast by `.to(output_dtype)` (NaN tangents stay NaN; their bit
+    pattern may differ).  Half the bytes of float32 to write, keep and copy.  Anything else raises ValueError."""
     if antialias_attr:
         raise NotImplementedError("antialias_attr=True (dr.antialias) is outside the geometry path")
     raw = render_geometry_raw(
@@ -440,7 +468,7 @@ def render(
         depth_normalization_strategy=depth_normalization_strategy,
         normal_background=normal_background, attr_background=attr_background, texture_override=texture_override,
         texture_filter_mode=texture_filter_mode, out_buffers=_out_buffers,
-        raster_done_event=_raster_done_event)
+        raster_done_event=_raster_done_event, output_dtype=output_dtype)
     out = RenderOutput(mask=raw["mask"], pos=raw["pos"], depth=raw.get("depth"), attr=raw.get("attr"),
                        normal=raw.get("normal"))
     out.tangent = raw.get("tangent")
