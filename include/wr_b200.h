@@ -71,6 +71,8 @@ int wr_version(void);
 
 /* One context per (device, stream in flight).  Not thread-safe, like the reference's contexts. */
 int wr_ctx_create(int device, wr_ctx **out);
+/* Waits for the device to finish the work in flight (kernels of the context's last calls may still read its scratch),
+ * then frees the scratch. */
 void wr_ctx_destroy(wr_ctx *ctx);
 /* bytes of device scratch currently held */
 uint64_t wr_ctx_scratch_bytes(const wr_ctx *ctx);

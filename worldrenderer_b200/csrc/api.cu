@@ -91,7 +91,10 @@ extern "C" void wr_ctx_destroy(wr_ctx *ctx)
         for (int i = 0; i <= WR_MAX_STAGES; ++i) cudaEventDestroy(ctx->marks[i]);
     if (ctx->scratch) {
         cudaSetDevice(ctx->device);
-        cudaFree(ctx->scratch);   // synchronises: nothing of this context is in flight afterwards
+        // The scratch comes from cudaMallocAsync, and cudaFree does not wait for such memory: kernels of this context's
+        // last calls may still read it (a context dropped right after a launch).  Wait for them, then free.
+        cudaDeviceSynchronize();
+        cudaFree(ctx->scratch);
     }
     free(ctx);
 }
@@ -113,7 +116,11 @@ int wr_scratch_reserve(wr_ctx *ctx, size_t bytes, cudaStream_t stream)
     ctx->clean_bytes = 0;
     if (ctx->scratch) {
         cudaError_t fe = cudaFreeAsync(ctx->scratch, stream);
-        if (fe != cudaSuccess) { cudaGetLastError(); cudaFree(ctx->scratch); }
+        if (fe != cudaSuccess) {  // cudaFree does not wait for stream-ordered memory: the stream's kernels may read it
+            cudaGetLastError();
+            cudaStreamSynchronize(stream);
+            cudaFree(ctx->scratch);
+        }
         ctx->scratch = nullptr;
         ctx->scratch_bytes = 0;
     }
